@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: the view-sharded training step of BASELINE.json.
 
-    python bench.py --gpus N --steps K --warmup W [--impl ours|reference|cpu]
+    python bench.py --gpus N --steps K --warmup W [--impl ours|reference|cpu] [--dump-outputs DIR]
 
 A "step" = forward + loss + backward of EVERY view of a 64-view 1080p batch over 1M SH3 Gaussians
 (config E of BASELINE.md; every view is config C), sharded round-robin over the N ranks, plus ONE
@@ -15,6 +15,9 @@ NCCL sum-allreduce of the flat gradient bucket when N > 1.  Total work is fixed 
   roofline       dominant kernel (blend backward, FP32-pipe bound): algorithmic flops / CUDA-event time,
                  against a live FFMA micro-benchmark; `stages` gives every stage against its own bound
   cpu_baseline   the CPU oracle port (oracle/rasterizer_oracle.c) on a bounded sample, N=1 rank 0 only
+
+--dump-outputs DIR writes what the last timed step returned (its loss and parameter gradients, for a fixed
+sample of Gaussians) as DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output.
 
 --impl reference runs the reference's OWN CUDA rasterizer (oracle/_ref, built unmodified from
 /root/reference) through the same Python wrapper and the same step loop on one GPU: the reference has
@@ -120,6 +123,23 @@ def measured_peaks():
         d = json.load(open(p))
         return float(d["hbm_gbs"]), "MEASURED_PEAKS.json (driver-measured copy bandwidth)"
     return 6650.0, "fallback of B200_PROFILING.md (MEASURED_PEAKS.json absent)"
+
+
+DUMP_GAUSSIANS = 65536  # Gaussians whose gradients --dump-outputs writes (15.5 MB at SH degree 3; the bucket is 236 MB)
+
+
+def dump_outputs(out_dir, params, host_loss):
+    """--dump-outputs: the loss of the last timed step and the gradient of every parameter tensor (the all-reduced
+    bucket the step returns) for the same seeded sample of Gaussians in every run, as float32 .npy files."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    idx = torch.randperm(params.P, generator=torch.Generator().manual_seed(0))[:DUMP_GAUSSIANS].sort().values
+    np.save(os.path.join(out_dir, "loss.npy"), host_loss.numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "gaussian_index.npy"), idx.numpy().astype(np.float64))
+    rows = idx.to(params.flat.device)
+    for n in params.names:
+        np.save(os.path.join(out_dir, f"grad_{n}.npy"), params.tensors[n].grad.index_select(0, rows).cpu().numpy().astype(np.float32))
 
 
 def get_api():
@@ -301,7 +321,7 @@ def run_cpu_sample(scene_cpu, cams_cpu, Wc_cpu, n_views):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps per leg (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "cpu"])
     ap.add_argument("--views", type=int, default=N_VIEWS)
@@ -311,7 +331,13 @@ def main():
     ap.add_argument("--host-threads", type=int, default=0, help="1: one host thread per stream (ours only)")
     ap.add_argument("--graphs", type=int, default=-1, help="1: per-view work replayed from CUDA graphs (GraphedStep); 0: launched kernel by kernel; "
                     "-1: graphs when a rank has at most 16 views (the host's launch rate matters when a step is short)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's loss and a fixed sample of its "
+                    "gradients to DIR/<name>.npy (ours only)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     a.warmup = max(a.warmup, 3) if a.impl != "cpu" else a.warmup
 
     if a.impl == "reference":
@@ -473,6 +499,8 @@ def main():
     clocks = sampler.stop() if rank_eff == 0 else None
     loss_value = float(host_loss.item())
     torch.cuda.synchronize()
+    if a.dump_outputs and rank_eff == 0:
+        dump_outputs(a.dump_outputs, params, host_loss)  # before anything below reuses the gradient bucket
     e2e_breakdown = {"upload_h2d_allgather_and_wait_for_previous_d2h_ms": round(marks["t0"].elapsed_time(marks["up"]), 4),
                      "step_ms": round(marks["up"].elapsed_time(marks["step"]), 4),
                      "download_d2h_ms": round(marks["step"].elapsed_time(marks["down"]), 4),

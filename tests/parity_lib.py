@@ -6,13 +6,22 @@ Parity levels (BASELINE.json north_star):
               n_contrib, final_T
   <= 1e-5   : colour, depth (max abs)
   <= 1e-4   : every gradient tensor (relative L2)
+
+The parity tests of tests/test_gpu_parity.py compare against stored records (`Recorded`,
+tests/golden/parity/*.npz) instead of a live build of the reference, so that they run from the
+repository alone.  A record keeps, per compared call, a SHA-256 digest of every bit-exact array and,
+for every array compared with a tolerance, the array itself when it is small, otherwise a fixed
+sample of it (`sample_index`) and its L2 norm.
 """
 from __future__ import annotations
 
+import hashlib
 import os
+import re
 import sys
 from typing import Dict, Optional
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -167,6 +176,216 @@ def compare_autograd(scene, cam, bg, Wc, Wd, scale_modifier=1.0, cov3D=None) -> 
             continue
         rep["grad_" + k] = rel_l2(ga, gb)
         rep["refspread_" + k] = rel_l2(b2["grads"][k], gb)
+    return rep
+
+
+# ---- stored records ----------------------------------------------------------------------------------
+
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden", "parity")
+RECORD_ENV = "BRS_RECORD_PARITY"  # a directory: write new records there instead of comparing
+FULL = 256  # tolerance-compared arrays up to this many elements are stored whole
+SAMPLE = 4096  # larger ones as this many elements at sample_index(n, SAMPLE)
+
+
+def sample_index(n: int, k: int) -> np.ndarray:
+    """k element indices spread over [0, n) by the golden-ratio sequence.  The first j indices of a sample
+    of k are the sample of j, so a stored sample can be shortened without being recorded again."""
+    j = np.arange(1, k + 1, dtype=np.float64)
+    return np.floor((j * 0.6180339887498949) % 1.0 * n).astype(np.int64)
+
+
+def digest(t: torch.Tensor) -> str:
+    """SHA-256 of dtype, shape and bytes (float -0.0 counted as 0.0, as `==` does)."""
+    t = t.detach()
+    if t.is_floating_point():
+        t = t + 0.0
+    a = t.contiguous().cpu().numpy()
+    h = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def floats(name: str, t: torch.Tensor) -> Dict[str, np.ndarray]:
+    """An array compared with a tolerance: whole when small, else its sample; and its L2 norm."""
+    a = t.detach().reshape(-1).float()
+    if a.numel() > FULL:
+        a = a[torch.from_numpy(sample_index(a.numel(), SAMPLE)).to(a.device)]
+    return {name: a.cpu().numpy(), name + ".norm": np.float64(t.detach().double().norm().item())}
+
+
+def rec_maxabs(mine, want, k, finite_only=False) -> float:
+    b = want[k].astype(np.float64)
+    a = mine[k][:b.size].astype(np.float64)
+    if finite_only:
+        ok = np.isfinite(b)
+        a, b = a[ok], b[ok]
+    return float(np.abs(a - b).max()) if b.size else 0.0
+
+
+def rec_rel_l2(mine, want, k) -> float:
+    """Relative L2 distance on the stored elements; never below the relative distance of the norms of the
+    whole arrays (|‖a‖ - ‖b‖| <= ‖a - b‖, so this adds no condition the full comparison would not)."""
+    b = want[k].astype(np.float64)
+    a = mine[k][:b.size].astype(np.float64)
+    nb = np.linalg.norm(b)
+    e = float(np.linalg.norm(a - b) / nb) if nb > 0 else float(np.linalg.norm(a))
+    n_want = float(want[k + ".norm"])
+    if n_want > 0:
+        e = max(e, abs(float(mine[k + ".norm"]) - n_want) / n_want)
+    return e
+
+
+def rec_mismatch(mine, want, k) -> int:
+    return int(str(want[k]) != str(mine[k]))
+
+
+class Recorded:
+    """The stored results of one test: `take(mine, reference)` returns the record of the test's next compared call.
+
+    With the environment variable BRS_RECORD_PARITY=<dir> the records are taken instead: `take` calls
+    `reference()`, which runs the reference's own CUDA build (oracle/_ref) on the same inputs, keeps and returns
+    its record, so that the test compares this library with the reference live; `finish` writes
+    <dir>/<test>.npz only when the test passed (tests/golden/make_golden_parity.py)."""
+
+    def __init__(self, test_name: str):
+        self.name = re.sub(r"[^A-Za-z0-9_.-]+", "-", test_name).strip("-")
+        self.out = os.environ.get(RECORD_ENV)
+        self.calls = []
+        self.pos = 0
+        if self.out:
+            assert reference() is not None, "recording needs the reference's own CUDA build (oracle/_ref/_ref_C.so)"
+        else:
+            path = os.path.join(GOLDEN_DIR, self.name + ".npz")
+            with np.load(path) as z:
+                data = {k: z[k] for k in z.files}
+            for i in range(int(data["calls"])):
+                p = f"c{i}."
+                self.calls.append({k[len(p):]: v for k, v in data.items() if k.startswith(p)})
+
+    def take(self, mine: Dict[str, object], reference_record) -> Dict[str, object]:
+        if self.out:
+            want = reference_record()
+            self.calls.append(want)
+        else:
+            assert self.pos < len(self.calls), f"{self.name}: more compared calls than stored records ({len(self.calls)})"
+            want = self.calls[self.pos]
+            self.pos += 1
+        assert set(want) == set(mine), (self.name, len(self.calls) - 1, sorted(set(want) ^ set(mine)))
+        return want
+
+    def finish(self, passed: bool):
+        if not passed:
+            return
+        if self.out:
+            os.makedirs(self.out, exist_ok=True)
+            d = {"calls": np.int64(len(self.calls))}
+            for i, rec in enumerate(self.calls):
+                d.update({f"c{i}.{k}": np.asarray(v) for k, v in rec.items()})
+            np.savez_compressed(os.path.join(self.out, self.name + ".npz"), **d)
+        else:
+            assert self.pos == len(self.calls), f"{self.name}: {len(self.calls) - self.pos} stored records were not compared"
+
+
+def _stage_record(R, color, depth, radii, P, views) -> Dict[str, object]:
+    """A forward reduced to what the stage comparison needs; `views()` gives its per-Gaussian, binning and
+    per-pixel arrays under common names (depth_bits, means2D, conic_opacity, tiles_touched, n_contrib, final_T,
+    point_list, ranges, sorted_keys)."""
+    rec = {"R": R, "radii": digest(radii), "visible": int((radii > 0).sum().item()), **floats("color", color)}
+    if P == 0:
+        return rec
+    rec.update(floats("depth", depth))
+    v = views()
+    vis = radii > 0
+    for k in ("depth_bits", "means2D", "conic_opacity"):
+        rec[k] = digest(v[k][vis])
+    for k in ("tiles_touched", "n_contrib", "final_T"):
+        rec[k] = digest(v[k])
+    if R > 0:
+        for k in ("point_list", "ranges", "sorted_keys"):
+            rec[k] = digest(v[k]) if isinstance(v[k], torch.Tensor) else v[k]
+    return rec
+
+
+def stage_record(scene, cam, bg, scale_modifier=1.0, cov3D=None) -> Dict[str, object]:
+    """This library's forward through the raw binding, reduced to what the stage comparison needs."""
+    from bloomscene_b200.debug import state_views
+
+    mine = ours()
+    R, color, depth, radii, geom, binning, img = mine._C.rasterize_gaussians(*forward_args(scene, cam, bg, scale_modifier, cov3D))
+    P, W, H = scene.P, cam.image_width, cam.image_height
+
+    def views():
+        sv = state_views(mine._C, geom, binning, img, P, R, W, H)
+        rect = sv["rect"]
+        v = {"depth_bits": sv["depth_key"], "means2D": sv["means2D"], "conic_opacity": sv["conic_opacity"],
+             "tiles_touched": ((rect[:, 0] >> 16) - (rect[:, 0] & 0xFFFF)) * ((rect[:, 1] >> 16) - (rect[:, 1] & 0xFFFF)),
+             "n_contrib": sv["n_contrib"], "final_T": sv["final_T"], "point_list": sv["point_list"], "ranges": sv["ranges"]}
+        # sorted 64-bit keys, reconstructed from (tile of the range, depth bits of the id)
+        starts, ends = sv["ranges"][:, 0].long(), sv["ranges"][:, 1].long()
+        tile_of = torch.repeat_interleave(torch.arange(starts.numel(), device=starts.device), (ends - starts).clamp(min=0))
+        v["sorted_keys"] = ((tile_of << 32) | (sv["depth_key"].long() & 0xFFFFFFFF)[sv["point_list"].long()]
+                            if tile_of.numel() == R else "ranges do not cover the point list")
+        return v
+
+    return _stage_record(R, color, depth, radii, P, views)
+
+
+def reference_stage_record(scene, cam, bg, scale_modifier=1.0, cov3D=None) -> Dict[str, object]:
+    """The same record of the reference's own CUDA build (its private buffers read through oracle/ref_state)."""
+    from oracle import ref_state
+
+    ref = reference()
+    R, color, depth, radii, geom, binning, img = ref._C.rasterize_gaussians(*forward_args(scene, cam, bg, scale_modifier, cov3D))
+    P, W, H = scene.P, cam.image_width, cam.image_height
+    ntiles = ((W + 15) // 16) * ((H + 15) // 16)
+
+    def views():
+        rg, ri = ref_state.geom_views(geom, P), ref_state.image_views(img, W, H)
+        v = {"depth_bits": rg["depths"].view(torch.int32), "means2D": rg["means2D"], "conic_opacity": rg["conic_opacity"],
+             "tiles_touched": rg["tiles_touched"], "n_contrib": ri["n_contrib"], "final_T": ri["accum_alpha"],
+             "ranges": ri["ranges"][:ntiles]}
+        if R > 0:
+            rb = ref_state.binning_views(binning, R)
+            v["point_list"], v["sorted_keys"] = rb["point_list"], rb["keys"]
+        return v
+
+    return _stage_record(R, color, depth, radii, P, views)
+
+
+def stages_vs_record(ref: Recorded, scene, cam, bg, scale_modifier=1.0, cov3D=None) -> Dict[str, object]:
+    """compare_stages against a stored record: a mismatch entry is 1 when the array differs anywhere."""
+    mine = stage_record(scene, cam, bg, scale_modifier, cov3D)
+    want = ref.take(mine, lambda: reference_stage_record(scene, cam, bg, scale_modifier, cov3D))
+    rep: Dict[str, object] = {"P": scene.P, "R_ours": mine["R"], "R_ref": int(want["R"]), "visible": int(want["visible"]),
+                              "radii_mismatch": rec_mismatch(mine, want, "radii"), "color_maxabs": rec_maxabs(mine, want, "color")}
+    if scene.P == 0:
+        return rep
+    for k in ("depth_bits", "means2D", "conic_opacity", "tiles_touched", "n_contrib", "final_T", "point_list", "ranges",
+              "sorted_keys"):
+        if k in want:
+            rep[k + "_mismatch"] = rec_mismatch(mine, want, k)
+    rep["depth_maxabs"] = rec_maxabs(mine, want, "depth")
+    return rep
+
+
+def autograd_record(api, scene, cam, bg, Wc, Wd, scale_modifier=1.0, cov3D=None) -> Dict[str, object]:
+    a = run_autograd(api, scene, cam, bg, Wc, Wd, scale_modifier, cov3D)
+    rec = {"radii": digest(a["radii"]), **floats("color", a["color"]), **floats("depth", a["depth"])}
+    for k, g in a["grads"].items():
+        if g is not None:
+            rec.update(floats("grad_" + k, g))
+    return rec
+
+
+def autograd_vs_record(ref: Recorded, scene, cam, bg, Wc, Wd, scale_modifier=1.0, cov3D=None) -> Dict[str, float]:
+    """compare_autograd against a stored record (gradients: relative L2 on the stored elements)."""
+    mine = autograd_record(ours(), scene, cam, bg, Wc, Wd, scale_modifier, cov3D)
+    want = ref.take(mine, lambda: autograd_record(reference(), scene, cam, bg, Wc, Wd, scale_modifier, cov3D))
+    rep = {"color_maxabs": rec_maxabs(mine, want, "color"), "depth_maxabs": rec_maxabs(mine, want, "depth"),
+           "radii_mismatch": rec_mismatch(mine, want, "radii")}
+    for k in want:
+        if k.startswith("grad_") and not k.endswith(".norm"):
+            rep[k] = rec_rel_l2(mine, want, k)
     return rep
 
 
