@@ -903,6 +903,13 @@ int brs_backward(const brs_view* view, const brs_gaussians* g, const int* radii,
                  const float* dL_dout_color, const float* dL_dout_depth, const brs_grads* grads, brs_alloc_fn alloc,
                  void* alloc_ctx, brs_stream stream)
 {
+	return brs_backward_ex(view, g, radii, state, dL_dout_color, dL_dout_depth, grads, nullptr, alloc, alloc_ctx, stream);
+}
+
+int brs_backward_ex(const brs_view* view, const brs_gaussians* g, const int* radii, const brs_fwd_state* state,
+                    const float* dL_dout_color, const float* dL_dout_depth, const brs_grads* grads,
+                    const brs_densify_stats* stats, brs_alloc_fn alloc, void* alloc_ctx, brs_stream stream)
+{
 	// reference: dL_dout_depth is plumbed and never used (backward.cu:443-554); it is read only when
 	// the caller opts in with brs_grads.depth_gradient
 	int st = validate_view(view, true);
@@ -912,6 +919,9 @@ int brs_backward(const brs_view* view, const brs_gaussians* g, const int* radii,
 	if (st != BRS_OK)
 		return st;
 	if (grads == nullptr || state == nullptr || alloc == nullptr)
+		return BRS_ERR_INVALID_ARG;
+	if (stats != nullptr && (stats->grad_norm == nullptr || stats->count == nullptr || stats->rows < 0 ||
+	                         (stats->index == nullptr && stats->rows < g->P)))
 		return BRS_ERR_INVALID_ARG;
 	const int P = g->P;
 	if (P == 0)
@@ -1019,6 +1029,12 @@ int brs_backward(const brs_view* view, const brs_gaussians* g, const int* radii,
 	pb.dL_dsh = M > 0 ? grads->dL_dsh : nullptr;
 	pb.dL_dscales = grads->dL_dscales;
 	pb.dL_drotations = grads->dL_drotations;
+	if (stats != nullptr) {
+		pb.stats_grad_norm = stats->grad_norm;
+		pb.stats_count = stats->count;
+		pb.stats_index = stats->index;
+		pb.stats_rows = stats->rows;
+	}
 	// (measured: moving this kernel to the companion stream as well is slightly slower)
 	BRS_STAGE(BRS_STAGE_PREPROCESS_BWD, launch_preprocess_backward(pb, stream), debug, stream);
 	return BRS_OK;

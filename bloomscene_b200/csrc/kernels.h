@@ -225,6 +225,11 @@ struct PreprocessBwdArgs {
 	float* dL_dsh;        // [P,M,3] or nullptr
 	float* dL_dscales;    // [P,3]
 	float* dL_drotations; // [P,4]
+	// optional densification statistics (brs_densify_stats); stats_grad_norm == nullptr: off
+	float* stats_grad_norm;       // [stats_rows] += |dL_dmeans2D[i, 0:2]| for radii[i] > 0
+	float* stats_count;           // [stats_rows] += 1 for the same Gaussians
+	const long long* stats_index; // [P] slot of Gaussian i (outside [0, stats_rows): skipped), or nullptr = identity
+	int stats_rows;
 };
 cudaError_t launch_preprocess_backward(const PreprocessBwdArgs& a, cudaStream_t stream);
 

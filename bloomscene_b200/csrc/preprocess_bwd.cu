@@ -44,7 +44,9 @@ constexpr int FACT_PITCH = 19; // 16 basis values + dL_dRGB, odd pitch -> confli
 
 // VEC / EAGER: as in the forward preprocess (preprocess.cu) - SH rows arrive by one bulk asynchronous copy per
 // lane, either for the whole warp at the very start (EAGER) or for the rendered Gaussians once `radii` is known.
-template <bool VEC, bool EAGER>
+// STATS: also add the densification statistics of this view (brs_densify_stats).  A template parameter, not a
+// runtime branch, so that the instantiations without it compile to the code they had before the option existed.
+template <bool VEC, bool EAGER, bool STATS>
 __global__ void __launch_bounds__(PB_THREADS, 6) preprocess_backward_kernel(PreprocessBwdArgs a)
 {
 	using namespace bwdmath;
@@ -242,6 +244,16 @@ __global__ void __launch_bounds__(PB_THREADS, 6) preprocess_backward_kernel(Prep
 		float* p;
 		p = a.dL_dmeans2D + 3 * (size_t)idx;
 		p[0] = o_m2x; p[1] = o_m2y; p[2] = 0.f;
+		if (STATS && visible) {
+			// reference scene/gaussian_model.py:756-759: norm of the per-view means2D gradient and one count per
+			// rendered Gaussian (also when that gradient is zero).  Float reductions: views on other streams add
+			// into the same accumulators concurrently.
+			const long long slot = a.stats_index != nullptr ? __ldg(a.stats_index + idx) : (long long)idx;
+			if (slot >= 0 && slot < a.stats_rows) {
+				atomicAdd(a.stats_grad_norm + slot, sqrtf(o_m2x * o_m2x + o_m2y * o_m2y));
+				atomicAdd(a.stats_count + slot, 1.0f);
+			}
+		}
 		if (!a.accumulate) {
 			p = a.dL_dcolors + 3 * (size_t)idx;
 			p[0] = o_color.x; p[1] = o_color.y; p[2] = o_color.z;
@@ -348,6 +360,15 @@ __global__ void __launch_bounds__(PB_THREADS, 6) preprocess_backward_kernel(Prep
 	}
 }
 
+template <bool VEC, bool EAGER>
+void launch_as(const PreprocessBwdArgs& args, int blocks, size_t smem, cudaStream_t stream)
+{
+	if (args.stats_grad_norm != nullptr)
+		preprocess_backward_kernel<VEC, EAGER, true><<<blocks, PB_THREADS, smem, stream>>>(args);
+	else
+		preprocess_backward_kernel<VEC, EAGER, false><<<blocks, PB_THREADS, smem, stream>>>(args);
+}
+
 } // namespace
 
 cudaError_t launch_preprocess_backward(const PreprocessBwdArgs& a, cudaStream_t stream)
@@ -367,11 +388,11 @@ cudaError_t launch_preprocess_backward(const PreprocessBwdArgs& a, cudaStream_t 
 	args.fact_offset = (int)(in / sizeof(float));
 	const size_t smem = in + (size_t)PB_THREADS * FACT_PITCH * sizeof(float);
 	if (vec && a.eager_sh)
-		preprocess_backward_kernel<true, true><<<blocks, PB_THREADS, smem, stream>>>(args);
+		launch_as<true, true>(args, blocks, smem, stream);
 	else if (vec)
-		preprocess_backward_kernel<true, false><<<blocks, PB_THREADS, smem, stream>>>(args);
+		launch_as<true, false>(args, blocks, smem, stream);
 	else
-		preprocess_backward_kernel<false, false><<<blocks, PB_THREADS, smem, stream>>>(args);
+		launch_as<false, false>(args, blocks, smem, stream);
 	count_launch();
 	return cudaGetLastError();
 }

@@ -277,7 +277,7 @@ void run_backward(const torch::Tensor& background, const torch::Tensor& means3D,
                   const torch::Tensor& dL_dout_color, const torch::Tensor& dL_dout_depth, const torch::Tensor& sh,
                   const int degree, const torch::Tensor& campos, const torch::Tensor& geomBuffer, const int R,
                   const torch::Tensor& binningBuffer, const torch::Tensor& imageBuffer, const bool debug, const int M,
-                  const brs_grads& grads_in, const char* what,
+                  const brs_grads& grads_in, const brs_densify_stats* stats, const char* what,
                   const c10::optional<torch::Tensor>& out_depth = c10::nullopt)
 {
 	brs_grads grads = grads_in;
@@ -338,8 +338,8 @@ void run_backward(const torch::Tensor& background, const torch::Tensor& means3D,
 	state.image_bytes = (size_t)img_c.numel();
 	state.num_rendered = R;
 
-	int st = brs_backward(&view, &g, radii_c.data_ptr<int>(), &state, dcol, ddepth, &grads, alloc_cb, &ctx,
-	                      current_stream());
+	int st = brs_backward_ex(&view, &g, radii_c.data_ptr<int>(), &state, dcol, ddepth, &grads, stats, alloc_cb, &ctx,
+	                         current_stream());
 	check_status(st, what);
 }
 
@@ -360,6 +360,39 @@ float* sink_ptr(const c10::optional<torch::Tensor>& t, int64_t numel, const char
 	return t->data_ptr<float>();
 }
 
+
+// Densification statistics of the backward bindings (brs_densify_stats): absent (all three None) -> nullptr.
+// grad_norm / count are caller-owned accumulators of any shape with the same number of elements (e.g. [rows, 1]),
+// updated in place; index, if given, maps each of the P Gaussians to its accumulator row.
+const brs_densify_stats* stats_of(const c10::optional<torch::Tensor>& grad_norm, const c10::optional<torch::Tensor>& count,
+                                  const c10::optional<torch::Tensor>& index, const torch::Tensor& means3D,
+                                  brs_densify_stats& out)
+{
+	auto given = [](const c10::optional<torch::Tensor>& t) { return t.has_value() && t->defined(); };
+	if (!given(grad_norm) && !given(count) && !given(index))
+		return nullptr;
+	TORCH_CHECK(given(grad_norm) && given(count), "densification statistics need both stats_grad_norm and stats_count");
+	for (const torch::Tensor* t : {&*grad_norm, &*count})
+		TORCH_CHECK(t->is_cuda() && t->device() == means3D.device() && t->scalar_type() == torch::kFloat32 && t->is_contiguous(),
+		            "stats_grad_norm / stats_count must be contiguous float32 tensors on the device of means3D");
+	TORCH_CHECK(grad_norm->numel() == count->numel(), "stats_grad_norm and stats_count must have the same number of elements");
+	TORCH_CHECK(grad_norm->numel() <= INT32_MAX, "densification statistics: more than 2^31 - 1 rows");
+	out = brs_densify_stats{};
+	out.grad_norm = grad_norm->data_ptr<float>();
+	out.count = count->data_ptr<float>();
+	out.rows = (int)grad_norm->numel();
+	if (given(index)) {
+		TORCH_CHECK(index->is_cuda() && index->device() == means3D.device() && index->scalar_type() == torch::kInt64 &&
+		                index->is_contiguous(),
+		            "stats_index must be a contiguous int64 tensor on the device of means3D");
+		TORCH_CHECK(index->numel() == means3D.size(0), "stats_index must have one entry per Gaussian");
+		out.index = reinterpret_cast<const long long*>(index->data_ptr<int64_t>());
+	} else {
+		TORCH_CHECK(out.rows >= means3D.size(0), "densification statistics without stats_index need at least P rows");
+	}
+	return &out;
+}
+
 } // namespace
 
 std::tuple<torch::Tensor, torch::Tensor, torch::Tensor, torch::Tensor, torch::Tensor, torch::Tensor, torch::Tensor,
@@ -373,12 +406,17 @@ RasterizeGaussiansBackwardImpl(const c10::optional<torch::Tensor>& out_depth, co
                                const torch::Tensor& dL_dout_color, const torch::Tensor& dL_dout_depth,
                                const torch::Tensor& sh, const int degree, const torch::Tensor& campos,
                                const torch::Tensor& geomBuffer, const int R, const torch::Tensor& binningBuffer,
-                               const torch::Tensor& imageBuffer, const bool debug)
+                               const torch::Tensor& imageBuffer, const bool debug,
+                               const c10::optional<torch::Tensor>& stats_grad_norm,
+                               const c10::optional<torch::Tensor>& stats_count,
+                               const c10::optional<torch::Tensor>& stats_index)
 {
 	TORCH_CHECK(means3D.is_cuda(), "means3D must be a CUDA tensor");
 	c10::cuda::CUDAGuard guard(means3D.device());
 	const int P = means3D.size(0);
 	const int M = sh_coeffs_of(sh);
+	brs_densify_stats stats_buf;
+	const brs_densify_stats* stats = stats_of(stats_grad_norm, stats_count, stats_index, means3D, stats_buf);
 
 	auto opts = means3D.options().dtype(torch::kFloat32);
 	torch::Tensor dL_dmeans3D = torch::empty({P, 3}, opts);
@@ -403,7 +441,7 @@ RasterizeGaussiansBackwardImpl(const c10::optional<torch::Tensor>& out_depth, co
 		grads.accumulate = 0;
 		run_backward(background, means3D, radii, colors, scales, rotations, scale_modifier, cov3D_precomp, viewmatrix,
 		             projmatrix, tan_fovx, tan_fovy, dL_dout_color, dL_dout_depth, sh, degree, campos, geomBuffer, R,
-		             binningBuffer, imageBuffer, debug, M, grads, "rasterize_gaussians_backward", out_depth);
+		             binningBuffer, imageBuffer, debug, M, grads, stats, "rasterize_gaussians_backward", out_depth);
 	}
 
 	return std::make_tuple(dL_dmeans2D, dL_dcolors, dL_dopacity, dL_dmeans3D, dL_dcov3D, dL_dsh, dL_dscales,
@@ -420,12 +458,14 @@ GradTuple RasterizeGaussiansBackwardCUDA(
     const torch::Tensor& cov3D_precomp, const torch::Tensor& viewmatrix, const torch::Tensor& projmatrix,
     const float tan_fovx, const float tan_fovy, const torch::Tensor& dL_dout_color, const torch::Tensor& dL_dout_depth,
     const torch::Tensor& sh, const int degree, const torch::Tensor& campos, const torch::Tensor& geomBuffer, const int R,
-    const torch::Tensor& binningBuffer, const torch::Tensor& imageBuffer, const bool debug)
+    const torch::Tensor& binningBuffer, const torch::Tensor& imageBuffer, const bool debug,
+    const c10::optional<torch::Tensor>& stats_grad_norm, const c10::optional<torch::Tensor>& stats_count,
+    const c10::optional<torch::Tensor>& stats_index)
 {
 	return RasterizeGaussiansBackwardImpl(c10::nullopt, background, means3D, radii, colors, scales, rotations,
 	                                      scale_modifier, cov3D_precomp, viewmatrix, projmatrix, tan_fovx, tan_fovy,
 	                                      dL_dout_color, dL_dout_depth, sh, degree, campos, geomBuffer, R, binningBuffer,
-	                                      imageBuffer, debug);
+	                                      imageBuffer, debug, stats_grad_norm, stats_count, stats_index);
 }
 
 // Extension (SURVEY.md 8f N3, opt-in): the same 22 arguments plus the forward's depth image; dL_dout_depth
@@ -436,12 +476,14 @@ GradTuple RasterizeGaussiansBackwardDepthCUDA(
     const torch::Tensor& cov3D_precomp, const torch::Tensor& viewmatrix, const torch::Tensor& projmatrix,
     const float tan_fovx, const float tan_fovy, const torch::Tensor& dL_dout_color, const torch::Tensor& dL_dout_depth,
     const torch::Tensor& sh, const int degree, const torch::Tensor& campos, const torch::Tensor& geomBuffer, const int R,
-    const torch::Tensor& binningBuffer, const torch::Tensor& imageBuffer, const bool debug, const torch::Tensor& out_depth)
+    const torch::Tensor& binningBuffer, const torch::Tensor& imageBuffer, const bool debug, const torch::Tensor& out_depth,
+    const c10::optional<torch::Tensor>& stats_grad_norm, const c10::optional<torch::Tensor>& stats_count,
+    const c10::optional<torch::Tensor>& stats_index)
 {
 	return RasterizeGaussiansBackwardImpl(out_depth, background, means3D, radii, colors, scales, rotations, scale_modifier,
 	                                      cov3D_precomp, viewmatrix, projmatrix, tan_fovx, tan_fovy, dL_dout_color,
 	                                      dL_dout_depth, sh, degree, campos, geomBuffer, R, binningBuffer, imageBuffer,
-	                                      debug);
+	                                      debug, stats_grad_norm, stats_count, stats_index);
 }
 
 // Extension (no reference counterpart): the same backward, but the parameter gradients are ADDED in
@@ -458,12 +500,16 @@ torch::Tensor RasterizeGaussiansBackwardAccumulateCUDA(
     const c10::optional<torch::Tensor>& sink_means3D, const c10::optional<torch::Tensor>& sink_colors,
     const c10::optional<torch::Tensor>& sink_opacity, const c10::optional<torch::Tensor>& sink_cov3D,
     const c10::optional<torch::Tensor>& sink_sh, const c10::optional<torch::Tensor>& sink_scales,
-    const c10::optional<torch::Tensor>& sink_rotations, const c10::optional<torch::Tensor>& out_depth)
+    const c10::optional<torch::Tensor>& sink_rotations, const c10::optional<torch::Tensor>& out_depth,
+    const c10::optional<torch::Tensor>& stats_grad_norm, const c10::optional<torch::Tensor>& stats_count,
+    const c10::optional<torch::Tensor>& stats_index)
 {
 	TORCH_CHECK(means3D.is_cuda(), "means3D must be a CUDA tensor");
 	c10::cuda::CUDAGuard guard(means3D.device());
 	const int64_t P = means3D.size(0);
 	const int M = sh_coeffs_of(sh);
+	brs_densify_stats stats_buf;
+	const brs_densify_stats* stats = stats_of(stats_grad_norm, stats_count, stats_index, means3D, stats_buf);
 	torch::Tensor dL_dmeans2D = torch::empty({P, 3}, means3D.options().dtype(torch::kFloat32));
 	if (P != 0) {
 		brs_grads grads{};
@@ -478,7 +524,7 @@ torch::Tensor RasterizeGaussiansBackwardAccumulateCUDA(
 		grads.accumulate = 1;
 		run_backward(background, means3D, radii, colors, scales, rotations, scale_modifier, cov3D_precomp, viewmatrix,
 		             projmatrix, tan_fovx, tan_fovy, dL_dout_color, dL_dout_depth, sh, degree, campos, geomBuffer, R,
-		             binningBuffer, imageBuffer, debug, M, grads, "rasterize_gaussians_backward_accumulate", out_depth);
+		             binningBuffer, imageBuffer, debug, M, grads, stats, "rasterize_gaussians_backward_accumulate", out_depth);
 	}
 	return dL_dmeans2D;
 }
@@ -843,11 +889,26 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m)
 	m.attr("FWD_AUTO") = (int)BRS_FWD_AUTO;
 	m.attr("FWD_EXACT") = (int)BRS_FWD_EXACT;
 	m.attr("FWD_DEFERRED") = (int)BRS_FWD_DEFERRED;
-	m.def("rasterize_gaussians_backward", &RasterizeGaussiansBackwardCUDA, pybind11::call_guard<pybind11::gil_scoped_release>());
-	m.def("rasterize_gaussians_backward_accumulate", &RasterizeGaussiansBackwardAccumulateCUDA,
+	// the reference's 22 backward arguments (positional, as it calls them), then each binding's own extras; the
+	// densification statistics (brs_densify_stats) are trailing keywords that default to None
+	using pybind11::arg;
+#define BRS_BWD_ARGS                                                                                                       \
+	arg("bg"), arg("means3D"), arg("radii"), arg("colors"), arg("scales"), arg("rotations"), arg("scale_modifier"),        \
+	    arg("cov3D_precomp"), arg("viewmatrix"), arg("projmatrix"), arg("tan_fovx"), arg("tan_fovy"), arg("dL_dout_color"), \
+	    arg("dL_dout_depth"), arg("sh"), arg("degree"), arg("campos"), arg("geomBuffer"), arg("R"), arg("binningBuffer"),  \
+	    arg("imageBuffer"), arg("debug")
+#define BRS_STATS_ARGS \
+	arg("stats_grad_norm") = pybind11::none(), arg("stats_count") = pybind11::none(), arg("stats_index") = pybind11::none()
+	m.def("rasterize_gaussians_backward", &RasterizeGaussiansBackwardCUDA, BRS_BWD_ARGS, BRS_STATS_ARGS,
 	      pybind11::call_guard<pybind11::gil_scoped_release>());
-	m.def("rasterize_gaussians_backward_depth", &RasterizeGaussiansBackwardDepthCUDA,
-	      pybind11::call_guard<pybind11::gil_scoped_release>());
+	m.def("rasterize_gaussians_backward_accumulate", &RasterizeGaussiansBackwardAccumulateCUDA, BRS_BWD_ARGS,
+	      arg("sink_means3D"), arg("sink_colors"), arg("sink_opacity"), arg("sink_cov3D"), arg("sink_sh"), arg("sink_scales"),
+	      arg("sink_rotations"), arg("out_depth"), BRS_STATS_ARGS, pybind11::call_guard<pybind11::gil_scoped_release>());
+	m.def("rasterize_gaussians_backward_depth", &RasterizeGaussiansBackwardDepthCUDA, BRS_BWD_ARGS, arg("out_depth"),
+	      BRS_STATS_ARGS, pybind11::call_guard<pybind11::gil_scoped_release>());
+#undef BRS_STATS_ARGS
+#undef BRS_BWD_ARGS
+	m.attr("HAS_DENSIFY_STATS") = true;
 	m.def("rasterize_aussians_filter", &RasterizeGaussiansfilterCUDA);
 	m.def("rasterize_gaussians_filter_compact", &RasterizeGaussiansfilterCompactCUDA);
 	m.def("mark_visible", &markVisible);

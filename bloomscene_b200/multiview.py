@@ -5,7 +5,9 @@ the full (replicated) Gaussian parameters, renders views `rank, rank+N, ...` of 
 rasterizer, and accumulates per-Gaussian parameter gradients locally.  The only exchange is ONE
 sum-allreduce of the flat fp32 gradient bucket per step (NCCL over NVLink on GPUs, gloo in the CPU
 tests).  `means2D` gradients and `radii` are per-view statistics (BloomScene's densification uses
-per-view norms, reference scene/gaussian_model.py:756-759) and are not reduced.
+per-view norms, reference scene/gaussian_model.py:756-759) and are not reduced; what densification derives
+from them (the per-Gaussian gradient-norm sum and count) rides in the bucket when the parameters carry
+slots for it (`GaussianParams(scene, densify_stats=True)`).
 
 The reference has no such mode (single process, one view per step: bloomscene.py:237-243); this is
 the data-parallel scaling axis BASELINE.json names.  The rasterizer class is injected so host-side
@@ -34,6 +36,11 @@ def view_sharded_step(params: GaussianParams, cameras: Sequence[Camera], bg: tor
     parameter gradients over ranks.  Returns the step loss (summed over all views), per-view radii
     counts and the number of views rendered locally.
 
+    When `params.densify` is set, `res["densify"]` = {"grad_norm": [P], "count": [P]}: the densification statistics
+    of this step's views (of all ranks after the all-reduce), views into the bucket valid until the next step.
+    The native rasterizer adds them in its backward kernel; any other rasterizer gets them from means2D.grad and
+    radii with the reference's torch statement.
+
     With the native rasterizer on a GPU the views are dealt round-robin onto `streams` CUDA streams: a
     view's preprocess / sort / binning kernels (small grids, latency- and bandwidth-bound) then run
     under another view's blend kernels (issue-bound), and the forward's one host wait for a view falls
@@ -47,6 +54,9 @@ def view_sharded_step(params: GaussianParams, cameras: Sequence[Camera], bg: tor
     use_sink = getattr(rasterizer_cls, "supports_grad_sink", False)
     n_lanes = max(1, min(streams, len(mine))) if (use_sink and dev.type == "cuda") else 1
     sink = params.grads() if use_sink else None
+    stats = params.densify
+    native_stats = stats is not None and getattr(rasterizer_cls, "supports_densify_stats", False)
+    extra = {"densify_stats": stats} if native_stats else {}
     losses = [torch.zeros((), dtype=torch.float32, device=dev) for _ in range(n_lanes)]
 
     zeroed = None
@@ -67,7 +77,8 @@ def view_sharded_step(params: GaussianParams, cameras: Sequence[Camera], bg: tor
     def one_view(vi: int, lane: int):
         cam = cameras[vi]
         settings = raster_settings(cam, params.sh_degree, bg, GaussianRasterizationSettings)
-        rast = rasterizer_cls(settings, grad_sink=sink) if sink is not None else rasterizer_cls(raster_settings=settings)
+        rast = (rasterizer_cls(settings, grad_sink=sink, **extra) if sink is not None
+                else rasterizer_cls(raster_settings=settings, **extra))
         means2D = params.zero_means2D().detach().requires_grad_(True)  # fresh leaf over a shared zero buffer
         color, radii, depth = rast(means3D=params.tensors["means3D"], means2D=means2D,
                                    opacities=params.tensors["opacities"], shs=params.get("shs"),
@@ -79,6 +90,13 @@ def view_sharded_step(params: GaussianParams, cameras: Sequence[Camera], bg: tor
             waited[lane] = True
         loss.backward()
         losses[lane] += loss.detach()
+        if stats is not None and not native_stats:
+            # reference scene/gaussian_model.py:756-759 (identity slot map)
+            with torch.no_grad():
+                update_filter = radii > 0
+                grad_norm = torch.norm(means2D.grad[update_filter, :2], dim=-1)
+                stats["grad_norm"][update_filter] += grad_norm
+                stats["count"][update_filter] += 1
         # per-view statistics for the caller's densification (reference scene/gaussian_model.py:742-759 reads
         # viewspace_points.grad[:, :2] and radii > 0 after every view)
         visible.append((vi, radii, means2D.grad if keep_means2D_grad else None))
@@ -123,7 +141,8 @@ def view_sharded_step(params: GaussianParams, cameras: Sequence[Camera], bg: tor
         dist.all_reduce(params.reduce_buffer(), op=dist.ReduceOp.SUM, group=group)
         loss_sum = params.loss_slot[0].clone()
     return {"loss": loss_sum, "views": mine, "radii": [(vi, r) for vi, r, _ in visible],
-            "means2D_grad": [(vi, m2) for vi, _, m2 in visible] if keep_means2D_grad else None}
+            "means2D_grad": [(vi, m2) for vi, _, m2 in visible] if keep_means2D_grad else None,
+            "densify": stats}
 
 
 class GraphedStep:
@@ -138,13 +157,18 @@ class GraphedStep:
 
     Capacity overflows of any view are OR-ed into one device word; it rides through the step's all-reduce as a
     count, so that every rank learns whether SOME rank overflowed and all of them repeat the step un-graphed
-    (exact sizes, marks raised) and re-capture.  All cameras must share resolution and field of view."""
+    (exact sizes, marks raised) and re-capture.  All cameras must share resolution and field of view.
+
+    When `params.densify` is set, every view (captured or in the un-graphed fallback) adds its densification
+    statistics there, and `res["densify"]` returns them as in `view_sharded_step`."""
 
     def __init__(self, params: GaussianParams, cameras: Sequence[Camera], bg: torch.Tensor, rasterizer_cls,
                  loss_fn: Callable[[torch.Tensor, torch.Tensor, Optional[torch.Tensor]], torch.Tensor],
                  rank: int = 0, world: int = 1, group=None, streams: int = 4, targets: Optional[torch.Tensor] = None):
         if not getattr(rasterizer_cls, "supports_deferred", False) or not getattr(rasterizer_cls, "supports_grad_sink", False):
             raise Exception("GraphedStep needs the native rasterizer (deferred forward + in-kernel gradient accumulation)")
+        if params.densify is not None and not getattr(rasterizer_cls, "supports_densify_stats", False):
+            raise Exception("GraphedStep: this rasterizer has no densification statistics")
         self.params, self.bg, self.rasterizer_cls, self.loss_fn = params, bg, rasterizer_cls, loss_fn
         self.rank, self.world, self.group = rank, world, group
         self.cameras = list(cameras)
@@ -171,7 +195,8 @@ class GraphedStep:
             image_height=c0.image_height, image_width=c0.image_width, tanfovx=c0.tanfovx, tanfovy=c0.tanfovy, bg=self.bg,
             scale_modifier=1.0, viewmatrix=lane["cam"][0:16].view(4, 4), projmatrix=lane["cam"][16:32].view(4, 4),
             sh_degree=p.sh_degree, campos=lane["cam"][32:35], prefiltered=False, debug=False)
-        rast = self.rasterizer_cls(settings, grad_sink=p.grads(), deferred_overflow=self.overflow)
+        extra = {} if p.densify is None else {"densify_stats": p.densify}
+        rast = self.rasterizer_cls(settings, grad_sink=p.grads(), deferred_overflow=self.overflow, **extra)
         means2D = p.zero_means2D().detach().requires_grad_(True)
         color, radii, depth = rast(means3D=p.tensors["means3D"], means2D=means2D, opacities=p.tensors["opacities"],
                                    shs=p.get("shs"), colors_precomp=p.get("colors_precomp"), scales=p.tensors["scales"],
@@ -245,7 +270,8 @@ class GraphedStep:
             res = self._plain()
             self._capture()
             return res
-        return {"loss": p.loss_slot[0].clone(), "views": self.mine, "radii": None, "means2D_grad": None}
+        return {"loss": p.loss_slot[0].clone(), "views": self.mine, "radii": None, "means2D_grad": None,
+                "densify": p.densify}
 
 
 _ZERO_STREAMS = {}

@@ -10,6 +10,7 @@ exercise identical Python on both sides.
 from __future__ import annotations
 
 from concurrent.futures import ThreadPoolExecutor
+from functools import partial
 from types import SimpleNamespace
 from typing import NamedTuple
 
@@ -94,7 +95,7 @@ def bind(_C) -> SimpleNamespace:
 
         @staticmethod
         def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                    raster_settings, grad_sink=None, depth_gradient=False, deferred_overflow=None):
+                    raster_settings, grad_sink=None, depth_gradient=False, deferred_overflow=None, densify_stats=None):
             rs = raster_settings
             args = (rs.bg, means3D, colors_precomp, opacities, scales, rotations, rs.scale_modifier, cov3Ds_precomp,
                     rs.viewmatrix, rs.projmatrix, rs.tanfovx, rs.tanfovy, rs.image_height, rs.image_width, sh,
@@ -109,6 +110,7 @@ def bind(_C) -> SimpleNamespace:
             num_rendered, color, depth, radii, geom, binning, image = out
             ctx.raster_settings = rs
             ctx.grad_sink = grad_sink
+            ctx.densify_stats = densify_stats
             ctx.num_rendered = num_rendered
             ctx.depth_gradient = bool(depth_gradient)
             # extension: with depth_gradient the backward also needs the depth image the forward produced
@@ -122,12 +124,17 @@ def bind(_C) -> SimpleNamespace:
             rs = ctx.raster_settings
             colors_precomp, means3D, scales, rotations, cov3Ds_precomp, radii, sh, geom, binning, image = ctx.saved_tensors[:10]
             out_depth = ctx.saved_tensors[10] if ctx.depth_gradient else None
+            # extension: the kernel adds this view's densification statistics into the caller's accumulators
+            ds = ctx.densify_stats
+            stats = {} if ds is None else {"stats_grad_norm": ds["grad_norm"], "stats_count": ds["count"],
+                                           "stats_index": ds.get("index")}
+            bw = lambda fn: partial(fn, **stats) if stats else fn
             if ctx.grad_sink is not None:
                 # extension: parameter gradients are added in place to the caller's sinks by the kernel
                 # (brs_grads.accumulate); autograd only carries the per-view means2D gradient
                 k = ctx.grad_sink
                 d_means2D = _guarded(
-                    _C.rasterize_gaussians_backward_accumulate,
+                    bw(_C.rasterize_gaussians_backward_accumulate),
                     (rs.bg, means3D, radii, colors_precomp, scales, rotations, rs.scale_modifier, cov3Ds_precomp,
                      rs.viewmatrix, rs.projmatrix, rs.tanfovx, rs.tanfovy, grad_out_color, grad_depth, sh, rs.sh_degree,
                      rs.campos, geom, ctx.num_rendered, binning, image, rs.debug,
@@ -135,20 +142,20 @@ def bind(_C) -> SimpleNamespace:
                      k.get("scales"), k.get("rotations"), out_depth),
                     rs.debug, "snapshot_bw.dump",
                     "\nAn error occured in backward. Writing snapshot_bw.dump for debugging.\n")
-                return None, d_means2D, None, None, None, None, None, None, None, None, None, None
+                return None, d_means2D, None, None, None, None, None, None, None, None, None, None, None
             if ctx.depth_gradient:
                 # extension: grad_depth is back-propagated through the depth image (default off = reference)
                 g = _guarded(
-                    _C.rasterize_gaussians_backward_depth,
+                    bw(_C.rasterize_gaussians_backward_depth),
                     (rs.bg, means3D, radii, colors_precomp, scales, rotations, rs.scale_modifier, cov3Ds_precomp,
                      rs.viewmatrix, rs.projmatrix, rs.tanfovx, rs.tanfovy, grad_out_color, grad_depth, sh, rs.sh_degree,
                      rs.campos, geom, ctx.num_rendered, binning, image, rs.debug, out_depth),
                     rs.debug, "snapshot_bw.dump",
                     "\nAn error occured in backward. Writing snapshot_bw.dump for debugging.\n")
                 d_means2D, d_colors, d_opacities, d_means3D, d_cov3D, d_sh, d_scales, d_rotations = g
-                return d_means3D, d_means2D, d_sh, d_colors, d_opacities, d_scales, d_rotations, d_cov3D, None, None, None, None
+                return d_means3D, d_means2D, d_sh, d_colors, d_opacities, d_scales, d_rotations, d_cov3D, None, None, None, None, None
             g = _guarded(
-                _C.rasterize_gaussians_backward,
+                bw(_C.rasterize_gaussians_backward),
                 (rs.bg, means3D, radii, colors_precomp, scales, rotations, rs.scale_modifier, cov3Ds_precomp,
                  rs.viewmatrix, rs.projmatrix, rs.tanfovx, rs.tanfovy, grad_out_color, grad_depth, sh, rs.sh_degree,
                  rs.campos, geom, ctx.num_rendered, binning, image, rs.debug),
@@ -157,16 +164,21 @@ def bind(_C) -> SimpleNamespace:
             d_means2D, d_colors, d_opacities, d_means3D, d_cov3D, d_sh, d_scales, d_rotations = g
             # one gradient per autograd input, in input order (reference __init__.py:144-154);
             # grad_radii carries nothing and grad_depth is plumbed down but unused by the kernels
-            return d_means3D, d_means2D, d_sh, d_colors, d_opacities, d_scales, d_rotations, d_cov3D, None, None, None, None
+            return d_means3D, d_means2D, d_sh, d_colors, d_opacities, d_scales, d_rotations, d_cov3D, None, None, None, None, None
 
     has_sink = hasattr(_C, "rasterize_gaussians_backward_accumulate")
     has_depth_grad = hasattr(_C, "rasterize_gaussians_backward_depth")
 
     has_deferred = hasattr(_C, "rasterize_gaussians_ex")
+    has_densify_stats = bool(getattr(_C, "HAS_DENSIFY_STATS", False))
 
     def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                            raster_settings, grad_sink=None, depth_gradient=False, deferred_overflow=None):
-        # reference __init__.py:21-42; `grad_sink` and `depth_gradient` are extensions (see GaussianRasterizer)
+                            raster_settings, grad_sink=None, depth_gradient=False, deferred_overflow=None,
+                            densify_stats=None):
+        # reference __init__.py:21-42; `grad_sink`, `depth_gradient`, `deferred_overflow` and `densify_stats` are
+        # extensions (see GaussianRasterizer)
+        if densify_stats is not None and not has_densify_stats:
+            raise Exception('this native module has no densification statistics')
         if depth_gradient and not has_depth_grad:
             raise Exception('this native module has no depth gradient (the reference comments it out)')
         if deferred_overflow is not None and not has_deferred:
@@ -180,7 +192,8 @@ def bind(_C) -> SimpleNamespace:
                 if t.numel() != 0 and t.requires_grad and name not in grad_sink:
                     raise Exception(f'grad_sink has no entry for {name}, whose gradient would be dropped')
         return _RasterizeGaussians.apply(means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
-                                         cov3Ds_precomp, raster_settings, grad_sink, depth_gradient, deferred_overflow)
+                                         cov3Ds_precomp, raster_settings, grad_sink, depth_gradient, deferred_overflow,
+                                         densify_stats)
 
     class GaussianRasterizer(nn.Module):
         """reference __init__.py:172-249: forward / visible_filter / markVisible with the same signatures.
@@ -195,13 +208,23 @@ def bind(_C) -> SimpleNamespace:
         gradient because every depth line of the reference's backward is commented out, backward.cu:443-554).
         With it, the gradient of the returned depth image flows back through D / acc (and its acc > 0.5
         gate, forward.cu:464-468) into opacities, means3D and scales / rotations | cov3D_precomp, so
-        BloomScene's depth losses (bloomscene.py:298-325) can act on the geometry."""
+        BloomScene's depth losses (bloomscene.py:298-325) can act on the geometry.
+
+        Extension: `densify_stats` (default None) = {"grad_norm": t, "count": t, "index": optional int64 [P]} of
+        caller-owned fp32 accumulators (any shape, same number of elements, e.g. [rows, 1]).  The backward then adds,
+        for every Gaussian i with radii[i] > 0, |means2D.grad[i, :2]| to grad_norm[slot] and 1 to count[slot], with
+        slot = index[i] (skipped outside [0, rows)) or i — what the densification statistics of Scaffold-GS
+        (training_statis, scene/gaussian_model.py:742-759) and 3DGS (add_densification_stats) compute from
+        means2D.grad and radii after every view, here without any per-view torch op, inside CUDA graphs and with
+        grad_sink."""
 
         supports_grad_sink = has_sink
         supports_depth_gradient = has_depth_grad
         supports_deferred = has_deferred
+        supports_densify_stats = has_densify_stats
 
-        def __init__(self, raster_settings, grad_sink=None, depth_gradient=False, deferred_overflow=None):
+        def __init__(self, raster_settings, grad_sink=None, depth_gradient=False, deferred_overflow=None,
+                     densify_stats=None):
             super().__init__()
             self.raster_settings = raster_settings
             self.grad_sink = grad_sink
@@ -210,6 +233,7 @@ def bind(_C) -> SimpleNamespace:
             # synchronisation in forward or backward, buffers sized from the high-water marks of the shape, capacity
             # overflows OR-ed into the tensor (non-zero = this forward's results are invalid, run it again without).
             self.deferred_overflow = deferred_overflow
+            self.densify_stats = densify_stats
 
         def markVisible(self, positions):
             rs = self.raster_settings
@@ -227,7 +251,7 @@ def bind(_C) -> SimpleNamespace:
             opt = lambda t: _absent() if t is None else t
             return rasterize_gaussians(means3D, means2D, opt(shs), opt(colors_precomp), opacities, opt(scales),
                                        opt(rotations), opt(cov3D_precomp), self.raster_settings, self.grad_sink,
-                                       self.depth_gradient, self.deferred_overflow)
+                                       self.depth_gradient, self.deferred_overflow, self.densify_stats)
 
         def visible_filter(self, means3D, scales=None, rotations=None, cov3D_precomp=None):
             rs = self.raster_settings

@@ -209,6 +209,30 @@ int brs_backward(const brs_view* view, const brs_gaussians* g, const int* radii,
                  const brs_grads* grads,
                  brs_alloc_fn alloc, void* alloc_ctx, brs_stream stream);
 
+/* Extension: densification statistics of one view, added by the backward itself.  The reference's callers read
+ * means2D.grad[:, :2] and radii > 0 after every view and add the gradient norm and a count into per-Gaussian
+ * accumulators (Scaffold-GS training_statis, scene/gaussian_model.py:742-759; 3DGS add_densification_stats).
+ * With `stats`, for every Gaussian i with radii[i] > 0 and slot s = index ? index[i] : i:
+ *   grad_norm[s] += sqrtf(gx*gx + gy*gy)   (gx, gy: the fp32 values written to dL_dmeans2D[i, 0:2])
+ *   count[s]     += 1                       (also when that gradient is zero)
+ * Slots outside [0, rows) are skipped (-1 = "no slot").  The additions are float reductions, so views running on
+ * different streams may add into the same accumulators at the same time; works in every brs_grads mode, after a
+ * DEFERRED forward and inside a CUDA graph.  The index type is that of brs_visible_filter_compact's `indices`. */
+typedef struct brs_densify_stats {
+	float* grad_norm;       /* [rows] */
+	float* count;           /* [rows] */
+	const long long* index; /* [P] slot of Gaussian i, or NULL = identity (then rows >= P is required) */
+	int rows;
+} brs_densify_stats;
+/* brs_backward plus optional densification statistics; stats == NULL is exactly brs_backward.  Returns
+ * BRS_ERR_INVALID_ARG, before any CUDA call, when grad_norm or count is NULL, rows < 0, or index is NULL and
+ * rows < P. */
+int brs_backward_ex(const brs_view* view, const brs_gaussians* g, const int* radii,
+                    const brs_fwd_state* state,
+                    const float* dL_dout_color, const float* dL_dout_depth,
+                    const brs_grads* grads, const brs_densify_stats* stats,
+                    brs_alloc_fn alloc, void* alloc_ctx, brs_stream stream);
+
 /* Replaces CudaRasterizer::Rasterizer::visible_filter (rasterizer.h:59-76, rasterizer_impl.cu:342-398):
  * radii only.  `scales_stride` is the row stride of `scales` in floats (3 when dense); BloomScene
  * passes a [:, :3] view of a [P,6] tensor (gaussian_renderer/__init__.py:344).  No allocations. */

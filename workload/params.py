@@ -18,21 +18,31 @@ class GaussianParams:
     Each parameter tensor is a leaf view into `flat`, and its `.grad` is preset to the matching view
     of `grad_bucket`, so every view's gradients land straight in the bucket (added by the kernel itself
     with the native rasterizer, by autograd otherwise) and a single allreduce covers all parameters
-    ((44 + 12 M) bytes per Gaussian, SURVEY.md §8e)."""
+    ((44 + 12 M) bytes per Gaussian, SURVEY.md §8e).
 
-    def __init__(self, scene: Scene):
+    `densify_stats=True` adds 2 P words to the all-reduced buffer, between the gradients and the loss / flag words:
+    `densify = {"grad_norm": [P], "count": [P]}`, the step's densification statistics (sum over this step's views
+    of |means2D.grad[i, :2]| and the number of views with radii[i] > 0).  They ride in the step's one all-reduce and
+    are cleared by `zero_grad()` like the gradients: per step, not running totals (a running total would be
+    multiplied by the world size at the next all-reduce), so callers add them into their own accumulators."""
+
+    def __init__(self, scene: Scene, densify_stats: bool = False):
         tensors = {k: v for k, v in scene.tensors().items()}
         self.names = [n for n in _ORDER if n in tensors]
         self.sh_degree = scene.sh_degree
         dev = scene.means3D.device
         sizes = [tensors[n].numel() for n in self.names]
-        self.flat = torch.empty(sum(sizes), dtype=torch.float32, device=dev)
-        # two extra words behind the gradients carry the step loss and a "some rank must repeat this step" count,
-        # so that a multi-rank step needs ONE collective
-        self._bucket_ext = torch.zeros(sum(sizes) + 2, dtype=torch.float32, device=dev)
-        self.grad_bucket = self._bucket_ext[:sum(sizes)]
-        self.loss_slot = self._bucket_ext[sum(sizes):sum(sizes) + 1]
-        self.flag_slot = self._bucket_ext[sum(sizes) + 1:]
+        G = sum(sizes)
+        S = 2 * tensors["means3D"].shape[0] if densify_stats else 0
+        self.flat = torch.empty(G, dtype=torch.float32, device=dev)
+        # two extra words behind the gradients (and the statistics) carry the step loss and a "some rank must repeat
+        # this step" count, so that a multi-rank step needs ONE collective
+        self._bucket_ext = torch.zeros(G + S + 2, dtype=torch.float32, device=dev)
+        self.grad_bucket = self._bucket_ext[:G]
+        self.densify = ({"grad_norm": self._bucket_ext[G:G + S // 2], "count": self._bucket_ext[G + S // 2:G + S]}
+                        if densify_stats else None)
+        self.loss_slot = self._bucket_ext[G + S:G + S + 1]
+        self.flag_slot = self._bucket_ext[G + S + 1:]
         self.tensors: Dict[str, torch.Tensor] = {}
         self._zero_means2D = None
         off = 0
@@ -52,7 +62,8 @@ class GaussianParams:
         self._bucket_ext.zero_()
 
     def reduce_buffer(self) -> torch.Tensor:
-        """What a multi-rank step all-reduces: the gradient bucket followed by the loss and the repeat-flag words."""
+        """What a multi-rank step all-reduces: the gradient bucket, the densification statistics if any, then the loss
+        and the repeat-flag words."""
         return self._bucket_ext
 
     def zero_means2D(self) -> torch.Tensor:
