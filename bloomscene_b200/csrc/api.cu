@@ -505,8 +505,10 @@ Caps caps_from_marks(const Marks& m)
 
 struct ForwardCtx {
 	const brs_view* view; // n_views of them
-	int n_views;          // > 1: a stack of views rendered as one pipeline (brs_forward_views)
-	int P, W, H;          // P: Gaussians per view; the pipeline works on n_views * P instances
+	int n_views;          // > 1: a stack of views rendered as one pipeline (brs_forward_views[_ex])
+	const int* view_P;    // Gaussians of each view (brs_forward_views_ex), or nullptr: every view sees all of them
+	size_t P_inst;        // instances (view, Gaussian) of the pipeline: the sum of view_P, else n_views * P
+	int W, H;
 	uint32_t grid_x, grid_y; // tiles of ONE view; the stack has n_views * grid_y tile rows
 	bool debug;
 	brs_alloc_fn alloc;
@@ -536,7 +538,7 @@ int enqueue_binning_and_blend(const ForwardCtx& c, const Caps& caps, uint32_t* r
 	c.state->binning = binning;
 	c.state->binning_bytes = binning_bytes(caps.R_cap);
 
-	const size_t P_inst = (size_t)c.P * c.n_views;          // instances: (view, Gaussian)
+	const size_t P_inst = c.P_inst;
 	const uint32_t rows = c.grid_y * (uint32_t)c.n_views;   // tile rows of the stack of views
 	BinPlan pl{};
 	pl.P = (uint32_t)P_inst;
@@ -610,15 +612,27 @@ int enqueue_binning_and_blend(const ForwardCtx& c, const Caps& caps, uint32_t* r
 	} else {
 		BRS_STAGE(BRS_STAGE_BLEND_FWD, launch_blend_forward(ba, stream), debug, stream);
 	}
+	if (c.view_P != nullptr) {
+		// a view without Gaussians comes out as the reference's P == 0 forward does: zeros, no background
+		const size_t npix = (size_t)c.W * c.H;
+		for (int v = 0; v < c.n_views; v++) {
+			if (c.view_P[v] == 0 && npix > 0) {
+				BRS_CUDA(cudaMemsetAsync(c.out_color + (size_t)v * NUM_CHANNELS * npix, 0, sizeof(float) * NUM_CHANNELS * npix, stream));
+				BRS_CUDA(cudaMemsetAsync(c.out_depth + (size_t)v * npix, 0, sizeof(float) * npix, stream));
+			}
+		}
+	}
 	return BRS_OK;
 }
 
-// One forward over a stack of n_views views of the same Gaussians (n_views == 1: brs_forward_ex).  The views'
-// preprocess launches write into ONE instance space — instance v * P + i is Gaussian i seen from view v, its
-// tile rectangle shifted down by v * grid_y rows — so that everything behind it (depth sort, emission, coarse
-// sort, fine binning, blend) runs once over all views.
-int forward_impl(const brs_view* views, int n_views, const brs_gaussians* g, float* out_color, float* out_depth, int* radii,
-                 brs_alloc_fn alloc, void* alloc_ctx, brs_fwd_state* state, const brs_fwd_options* opt, cudaStream_t stream)
+// One forward over a stack of n_views views (n_views == 1: brs_forward_ex).  The views' preprocess launches write
+// into ONE instance space — with view_P == nullptr instance v * P + i is Gaussian i seen from view v, else view v
+// owns rows and instances [off_v, off_v + view_P[v]) — each instance's tile rectangle shifted down by v * grid_y
+// rows, so that everything behind it (depth sort, emission, coarse sort, fine binning, blend) runs once over all
+// views.
+int forward_impl(const brs_view* views, int n_views, const brs_gaussians* g, const int* view_P, float* out_color,
+                 float* out_depth, int* radii, brs_alloc_fn alloc, void* alloc_ctx, brs_fwd_state* state,
+                 const brs_fwd_options* opt, cudaStream_t stream)
 {
 	const brs_view* view = views;
 	if (views == nullptr || n_views < 1 || n_views > 65535)
@@ -636,6 +650,18 @@ int forward_impl(const brs_view* views, int n_views, const brs_gaussians* g, flo
 	}
 	if (st != BRS_OK)
 		return st;
+	if (view_P != nullptr) {
+		long long sum = 0;
+		for (int v = 0; v < n_views; v++) {
+			if (view_P[v] < 0)
+				return BRS_ERR_INVALID_ARG;
+			sum += view_P[v];
+		}
+		if (sum > (1ll << 31) - 1)
+			return BRS_ERR_UNSUPPORTED; // instance ids are 32-bit
+		if (sum != g->P)
+			return BRS_ERR_INVALID_ARG;
+	}
 	if (alloc == nullptr || state == nullptr)
 		return BRS_ERR_INVALID_ARG;
 	static const bool nvtx_env = [] {
@@ -652,7 +678,7 @@ int forward_impl(const brs_view* views, int n_views, const brs_gaussians* g, flo
 		return BRS_ERR_INVALID_ARG;
 	const int W = view->image_width, H = view->image_height, P = g->P;
 	const size_t npix = (size_t)W * H * n_views;
-	const size_t P_inst = (size_t)P * n_views;
+	const size_t P_inst = view_P != nullptr ? (size_t)P : (size_t)P * n_views;
 	if (P_inst > (1ull << 31) - 1 || (size_t)((H + TILE_Y - 1) / TILE_Y) * n_views >= 65536)
 		return BRS_ERR_UNSUPPORTED; // instance ids are 32-bit, tile rows of the stack are packed into 16 bits
 	if ((npix > 0 && (out_color == nullptr || out_depth == nullptr)) || (P > 0 && radii == nullptr))
@@ -676,7 +702,8 @@ int forward_impl(const brs_view* views, int n_views, const brs_gaussians* g, flo
 	ForwardCtx c{};
 	c.view = view;
 	c.n_views = n_views;
-	c.P = P;
+	c.view_P = view_P;
+	c.P_inst = P_inst;
 	c.W = W;
 	c.H = H;
 	c.grid_x = (W + TILE_X - 1) / TILE_X;
@@ -744,7 +771,9 @@ int forward_impl(const brs_view* views, int n_views, const brs_gaussians* g, flo
 		pa.row_offset = 0;
 		BRS_STAGE(BRS_STAGE_PREPROCESS, launch_preprocess(pa, stream), debug, stream);
 	} else {
-		// one launch per 16 views: blockIdx.y picks the view, its outputs go to instances [v * P, (v + 1) * P)
+		// one launch per 16 views: blockIdx.y picks the view, its outputs go to instances [v * P, (v + 1) * P), or
+		// with view_P to [off_v, off_v + view_P[v]), where off_v is also its first input row
+		size_t off = 0;
 		for (int v0 = 0; v0 < n_views; v0 += PreprocessViewTable::MAX_VIEWS) {
 			const int nv = n_views - v0 < PreprocessViewTable::MAX_VIEWS ? n_views - v0 : PreprocessViewTable::MAX_VIEWS;
 			PreprocessViewTable t{};
@@ -761,6 +790,10 @@ int forward_impl(const brs_view* views, int n_views, const brs_gaussians* g, flo
 				sl.focal_x = W / (2.0f * vw->tanfovx);
 				sl.scale_modifier = vw->scale_modifier;
 				sl.prefiltered = vw->prefiltered;
+				sl.count = (uint32_t)(view_P != nullptr ? view_P[v0 + k] : P);
+				sl.row = view_P != nullptr ? (uint32_t)off : 0u;
+				sl.inst = (uint32_t)off;
+				off += sl.count;
 			}
 			BRS_STAGE(BRS_STAGE_PREPROCESS, launch_preprocess_stack(pa, t, nv, stream), debug, stream);
 		}
@@ -847,15 +880,23 @@ int brs_forward(const brs_view* view, const brs_gaussians* g, float* out_color, 
 int brs_forward_ex(const brs_view* view, const brs_gaussians* g, float* out_color, float* out_depth, int* radii,
                    brs_alloc_fn alloc, void* alloc_ctx, brs_fwd_state* state, const brs_fwd_options* opt, brs_stream stream)
 {
-	return forward_impl(view, 1, g, out_color, out_depth, radii, alloc, alloc_ctx, state, opt, stream);
+	return forward_impl(view, 1, g, nullptr, out_color, out_depth, radii, alloc, alloc_ctx, state, opt, stream);
 }
 
 int brs_forward_views(const brs_view* views, int n_views, const brs_gaussians* g, float* out_color, float* out_depth,
                       int* radii, brs_alloc_fn alloc, void* alloc_ctx, long long* num_rendered, const brs_fwd_options* opt,
                       brs_stream stream)
 {
+	return brs_forward_views_ex(views, n_views, g, nullptr, out_color, out_depth, radii, alloc, alloc_ctx, num_rendered, opt,
+	                            stream);
+}
+
+int brs_forward_views_ex(const brs_view* views, int n_views, const brs_gaussians* g, const int* view_P, float* out_color,
+                         float* out_depth, int* radii, brs_alloc_fn alloc, void* alloc_ctx, long long* num_rendered,
+                         const brs_fwd_options* opt, brs_stream stream)
+{
 	brs_fwd_state st{};
-	const int rc = forward_impl(views, n_views, g, out_color, out_depth, radii, alloc, alloc_ctx, &st, opt, stream);
+	const int rc = forward_impl(views, n_views, g, view_P, out_color, out_depth, radii, alloc, alloc_ctx, &st, opt, stream);
 	if (num_rendered != nullptr)
 		*num_rendered = st.num_rendered;
 	return rc;

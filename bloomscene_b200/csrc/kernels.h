@@ -36,9 +36,12 @@ struct PreprocessArgs {
 	uint32_t* total_tiles; // [5], pre-zeroed: R = tile instances, R1 = supertile instances, max(~depth bits),
 	                       // max(depth bits) over visible, V = number of visible Gaussians
 };
-cudaError_t launch_preprocess(const PreprocessArgs& a, cudaStream_t stream);
+cudaError_t launch_preprocess(const PreprocessArgs& a, cudaStream_t stream); // one view of a.P Gaussians
 // Up to MAX_VIEWS views of a stack in one launch: the per-view fields of PreprocessArgs come from the table,
-// view k of the launch is view first_view + k of the stack (row offset, output slices).
+// view k of the launch is view first_view + k of the stack (tile row offset).  View k reads input rows
+// [row, row + count) and writes instances [inst, inst + count); PreprocessArgs::P is not read by the kernel.
+// A single view is the table {(0, 0, P)}, a stack of one Gaussian set {(0, v * P, P)}, a stack whose views
+// own consecutive rows of concatenated inputs (brs_forward_views_ex) {(off_v, off_v, P_v)}.
 struct PreprocessViewTable {
 	static constexpr int MAX_VIEWS = 16;
 	struct Slot {
@@ -47,6 +50,7 @@ struct PreprocessViewTable {
 		const float* campos;
 		float tan_fovx, tan_fovy, focal_x, focal_y, scale_modifier;
 		int prefiltered;
+		uint32_t row, inst, count; // first input row, first instance, Gaussians of this view (sum over a stack < 2^31)
 	} v[MAX_VIEWS];
 	uint32_t first_view;
 };

@@ -361,16 +361,31 @@ __device__ __forceinline__ void preprocess_body(const PreprocessArgs& a)
 	}
 }
 
-// One view, or a stack of views in ONE launch (brs_forward_views): blockIdx.y picks the view; its camera, its
-// place in the stack (row offset) and its slice of the instance-indexed outputs come from the view table in
-// parameter space.  The Gaussians' inputs are read once per view, the later views' reads hitting L2.
-// A single view runs the same kernel with a one-entry table, so a stacked forward and per-view forwards execute
-// the same instructions (two separately compiled copies of the SH evaluation differed in the last bit).
+// Offsets an optional input (nullptr = absent, which preprocess_body tests) to the view's first row.
+__device__ __forceinline__ const float* view_rows(const float* p, size_t floats) { return p != nullptr ? p + floats : p; }
+
+// One view, or a stack of views in ONE launch (brs_forward_views[_ex]): blockIdx.y picks the view; its camera, its
+// place in the stack (tile row offset), its input rows and its slice of the instance-indexed outputs come from the
+// view table in parameter space.  When the views share one Gaussian set, its inputs are read once per view, the
+// later views' reads hitting L2.  A single view runs the same kernel with a one-entry table, so a stacked forward
+// and per-view forwards execute the same instructions (two separately compiled copies of the SH evaluation
+// differed in the last bit).  The grid has ceil(max count / PRE_THREADS) blocks in x: blocks past their view's
+// count leave before they touch anything (shared memory, barriers, the header atomics).
 template <bool VEC, bool EAGER>
 __global__ void __launch_bounds__(PRE_THREADS) preprocess_kernel(PreprocessArgs a, PreprocessViewTable t)
 {
 	const PreprocessViewTable::Slot& v = t.v[blockIdx.y];
-	const size_t first = (size_t)(t.first_view + blockIdx.y) * (size_t)a.P;
+	if (blockIdx.x * PRE_THREADS >= v.count)
+		return;
+	const size_t row = v.row, first = v.inst;
+	a.P = (int)v.count;
+	a.means3D += 3 * row;
+	a.scales = view_rows(a.scales, 3 * row);
+	a.rotations = view_rows(a.rotations, 4 * row);
+	a.opacities += row;
+	a.shs = view_rows(a.shs, (size_t)(3 * a.M) * row);
+	a.cov3D_precomp = view_rows(a.cov3D_precomp, 6 * row);
+	a.colors_precomp = view_rows(a.colors_precomp, 3 * row);
 	a.viewmatrix = v.viewmatrix;
 	a.projmatrix = v.projmatrix;
 	a.campos = v.campos;
@@ -518,16 +533,27 @@ cudaError_t launch_preprocess(const PreprocessArgs& a, cudaStream_t stream)
 	s.focal_y = a.focal_y;
 	s.scale_modifier = a.scale_modifier;
 	s.prefiltered = a.prefiltered;
+	s.row = 0;
+	s.inst = 0;
+	s.count = a.P < 0 ? 0u : (uint32_t)a.P;
 	return launch_preprocess_stack(a, t, 1, stream);
 }
 
+// The grid is sized by the largest view of the launch (not a flat grid over all rows with a per-block search of
+// the table): the block -> (view, row) map stays blockIdx.y / blockIdx.x * PRE_THREADS as for a single view, at
+// the price of blocks that exit at once in the shorter views of a ragged stack.
 cudaError_t launch_preprocess_stack(const PreprocessArgs& a, const PreprocessViewTable& t, int n_views, cudaStream_t stream)
 {
-	if (a.P <= 0 || n_views <= 0)
+	if (n_views <= 0)
 		return cudaSuccess;
 	if (n_views > PreprocessViewTable::MAX_VIEWS)
 		return cudaErrorInvalidValue;
-	const dim3 grid((a.P + PRE_THREADS - 1) / PRE_THREADS, n_views, 1);
+	uint32_t max_count = 0;
+	for (int k = 0; k < n_views; k++)
+		max_count = t.v[k].count > max_count ? t.v[k].count : max_count;
+	if (max_count == 0)
+		return cudaSuccess;
+	const dim3 grid((max_count + PRE_THREADS - 1) / PRE_THREADS, n_views, 1);
 	size_t smem = 0;
 	bool vec = false;
 	if (a.shs != nullptr) {

@@ -184,6 +184,8 @@ ForwardTuple RasterizeGaussiansCUDA(const torch::Tensor& background, const torch
 // Extension (brs_forward_views): n views of the same Gaussians as ONE pipeline, forward only.
 // viewmatrices / projmatrices [n,4,4], camposes [n,3], tan_fovx / tan_fovy one value per view (or one for all).
 // Returns (instances of all views, color [n,3,H,W], depth [n,1,H,W], radii [n,P]).
+// With `view_counts` (brs_forward_views_ex) view v renders its own rows [off_v, off_v + view_counts[v]) of the
+// concatenated inputs instead, and radii is [P] in row order.
 std::tuple<int64_t, torch::Tensor, torch::Tensor, torch::Tensor>
 RasterizeGaussiansViewsCUDA(const torch::Tensor& background, const torch::Tensor& means3D, const torch::Tensor& colors,
                             const torch::Tensor& opacity, const torch::Tensor& scales, const torch::Tensor& rotations,
@@ -192,7 +194,7 @@ RasterizeGaussiansViewsCUDA(const torch::Tensor& background, const torch::Tensor
                             const std::vector<double>& tan_fovy, const int image_height, const int image_width,
                             const torch::Tensor& sh, const int degree, const torch::Tensor& camposes, const bool prefiltered,
                             const bool debug, const int mode, const c10::optional<torch::Tensor>& color_out,
-                            const c10::optional<torch::Tensor>& depth_out)
+                            const c10::optional<torch::Tensor>& depth_out, const c10::optional<std::vector<int64_t>>& view_counts)
 {
 	TORCH_CHECK(means3D.ndimension() == 2 && means3D.size(1) == 3, "means3D must have dimensions (num_points, 3)");
 	TORCH_CHECK(means3D.is_cuda(), "means3D must be a CUDA tensor");
@@ -218,7 +220,19 @@ RasterizeGaussiansViewsCUDA(const torch::Tensor& background, const torch::Tensor
 	};
 	torch::Tensor out_color = take(color_out, 3, "color_out");
 	torch::Tensor out_depth = take(depth_out, 1, "depth_out");
-	torch::Tensor radii = torch::empty({n, P}, means3D.options().dtype(torch::kInt32));
+	std::vector<int> counts;
+	if (view_counts.has_value()) {
+		TORCH_CHECK((int)view_counts->size() == n, "view_counts must have one entry per view");
+		int64_t sum = 0;
+		for (int64_t c : *view_counts) {
+			TORCH_CHECK(c >= 0, "view_counts must not be negative");
+			sum += c;
+		}
+		TORCH_CHECK(sum == P, "view_counts must add up to the rows of means3D");
+		counts.assign(view_counts->begin(), view_counts->end());
+	}
+	torch::Tensor radii = view_counts.has_value() ? torch::empty({P}, means3D.options().dtype(torch::kInt32))
+	                                              : torch::empty({n, P}, means3D.options().dtype(torch::kInt32));
 
 	AllocCtx ctx;
 	ctx.byte_opts = torch::TensorOptions(torch::kByte).device(means3D.device());
@@ -261,8 +275,9 @@ RasterizeGaussiansViewsCUDA(const torch::Tensor& background, const torch::Tensor
 	brs_fwd_options opt{};
 	opt.mode = mode;
 	long long R = 0;
-	int st = brs_forward_views(views.data(), n, &g, out_color.data_ptr<float>(), out_depth.data_ptr<float>(),
-	                           P ? radii.data_ptr<int>() : nullptr, alloc_cb, &ctx, &R, &opt, current_stream());
+	int st = brs_forward_views_ex(views.data(), n, &g, view_counts.has_value() ? counts.data() : nullptr,
+	                              out_color.data_ptr<float>(), out_depth.data_ptr<float>(), P ? radii.data_ptr<int>() : nullptr,
+	                              alloc_cb, &ctx, &R, &opt, current_stream());
 	check_status(st, "rasterize_gaussians_views");
 	return std::make_tuple((int64_t)R, out_color, out_depth, radii);
 }
@@ -861,7 +876,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m)
 	      pybind11::arg("projmatrices"), pybind11::arg("tan_fovx"), pybind11::arg("tan_fovy"), pybind11::arg("image_height"),
 	      pybind11::arg("image_width"), pybind11::arg("sh"), pybind11::arg("degree"), pybind11::arg("camposes"),
 	      pybind11::arg("prefiltered"), pybind11::arg("debug"), pybind11::arg("mode") = (int)BRS_FWD_AUTO,
-	      pybind11::arg("color_out") = c10::nullopt, pybind11::arg("depth_out") = c10::nullopt);
+	      pybind11::arg("color_out") = c10::nullopt, pybind11::arg("depth_out") = c10::nullopt,
+	      pybind11::arg("view_counts") = c10::nullopt);
 	m.def("rasterize_gaussians_ex", &RasterizeGaussiansExCUDA, pybind11::arg("bg"), pybind11::arg("means3D"), pybind11::arg("colors"),
 	      pybind11::arg("opacity"), pybind11::arg("scales"), pybind11::arg("rotations"), pybind11::arg("scale_modifier"),
 	      pybind11::arg("cov3D_precomp"), pybind11::arg("viewmatrix"), pybind11::arg("projmatrix"), pybind11::arg("tan_fovx"),

@@ -276,7 +276,8 @@ def bind(_C) -> SimpleNamespace:
                 return radii, idx[: int(count.item())]
 
     def render_views(raster_settings_list, means3D, opacities, shs=None, colors_precomp=None, scales=None,
-                     rotations=None, cov3D_precomp=None, streams=4, keep_radii=False, host_threads=True, stack=0):
+                     rotations=None, cov3D_precomp=None, streams=4, keep_radii=False, host_threads=True, stack=0,
+                     view_counts=None):
         """Forward-only render of one Gaussian set from a list of cameras (BloomScene's render_video loop,
         reference bloomscene.py:191-204, one `GaussianRasterizer` call per frame there).  Extension: no
         autograd graph, no saved state, and on a GPU the views are dealt onto `streams` CUDA streams so that
@@ -291,7 +292,15 @@ def bind(_C) -> SimpleNamespace:
         preprocess launch per view into a shared instance space, then one depth sort, one emission / coarse sort /
         fine binning and one blend launch for the whole stack, at most one host wait per stack; the stacks are
         dealt onto `streams` lanes (streams=1: everything on the caller's stream).  Same bits as the per-view path.  Views of a stack must share background, scale modifier and flags
-        (a run of views that does not is cut into shorter stacks)."""
+        (a run of views that does not is cut into shorter stacks).
+
+        `view_counts` (a list of B ints, default None = every view renders all rows): every view renders its OWN
+        Gaussians, as BloomScene's render loop does (each frame culls anchors and generates its own neural
+        Gaussians, reference bloomscene.py:174-219).  The attribute tensors then hold the views' rows concatenated
+        in view order, view j owning the next view_counts[j] rows, and every view's result is bit-identical to a
+        single `GaussianRasterizer` call on its own rows (a view with 0 rows gives zeros, without background, as
+        that call does).  Stacks go through `brs_forward_views_ex`; the per-view route slices each view's rows.
+        With `keep_radii` the radii list holds one [view_counts[j]] tensor per view."""
         views = list(raster_settings_list)
         if (shs is None) == (colors_precomp is None):
             raise Exception('Please provide excatly one of either SHs or precomputed colors!')
@@ -301,12 +310,28 @@ def bind(_C) -> SimpleNamespace:
         opt = lambda t: _absent() if t is None else t.detach()
         dev = means3D.device
         B = len(views)
+        counts = None
+        if view_counts is not None:
+            counts = [int(c) for c in view_counts]
+            if len(counts) != B or min(counts, default=0) < 0 or sum(counts) != means3D.shape[0]:
+                raise Exception('render_views: view_counts must give every view a non-negative row count, '
+                                'adding up to the rows of means3D')
+        offs = [0]
+        for c in counts or []:
+            offs.append(offs[-1] + c)
         H, W = (views[0].image_height, views[0].image_width) if B else (0, 0)
         color = torch.empty((B, 3, H, W), dtype=torch.float32, device=dev)
         depth = torch.empty((B, 1, H, W), dtype=torch.float32, device=dev)
         radii = [None] * B if keep_radii else None
         m3, op = means3D.detach(), opacities.detach()
         sh_, cp_, sc_, ro_, cv_ = opt(shs), opt(colors_precomp), opt(scales), opt(rotations), opt(cov3D_precomp)
+        attrs = (m3, op, sh_, cp_, sc_, ro_, cv_)
+
+        def rows(j, n=1):
+            """The inputs of views j .. j + n - 1: all rows, or with view_counts their rows (absent inputs stay)."""
+            if counts is None:
+                return attrs
+            return tuple(t if t.numel() == 0 else t[offs[j]:offs[j + n]] for t in attrs)
 
         # Native module with brs_fwd_options: every view is a DEFERRED forward (no host wait at all; buffers sized
         # from the high-water marks of this shape); the instance counts land in pinned host memory and are
@@ -318,8 +343,11 @@ def bind(_C) -> SimpleNamespace:
         def one(j, rs, exact=False):
             if (rs.image_height, rs.image_width) != (H, W):
                 raise Exception('render_views: all views of a batch must share one resolution')
-            args = (rs.bg, m3, cp_, op, sc_, ro_, rs.scale_modifier, cv_, rs.viewmatrix, rs.projmatrix, rs.tanfovx,
-                    rs.tanfovy, rs.image_height, rs.image_width, sh_, rs.sh_degree, rs.campos, rs.prefiltered, rs.debug)
+            v_m3, v_op, v_sh, v_cp, v_sc, v_ro, v_cv = rows(j)
+            args = (rs.bg, v_m3, v_cp, v_op, v_sc, v_ro, rs.scale_modifier, v_cv, rs.viewmatrix, rs.projmatrix, rs.tanfovx,
+                    rs.tanfovy, rs.image_height, rs.image_width, v_sh, rs.sh_degree, rs.campos, rs.prefiltered, rs.debug)
+            if deferred and counts is not None and not _C.has_marks(counts[j], W, H):
+                exact = True  # views with their own rows: a row count never seen before seeds its high-water marks
             if deferred and not exact:
                 out = _C.rasterize_gaussians_ex(*args, _C.FWD_DEFERRED, 0, 0, 0, reports[j])
             elif deferred:
@@ -351,13 +379,16 @@ def bind(_C) -> SimpleNamespace:
                 vm = torch.stack([v.viewmatrix for v in grp])
                 pm = torch.stack([v.projmatrix for v in grp])
                 cps = torch.stack([v.campos for v in grp])
+                s_m3, s_op, s_sh, s_cp, s_sc, s_ro, s_cv = rows(j, n)
+                extra = {} if counts is None else {"view_counts": counts[j:j + n]}
                 _, _, _, r = _C.rasterize_gaussians_views(
-                    rs.bg, m3, cp_, op, sc_, ro_, rs.scale_modifier, cv_, vm, pm, [float(v.tanfovx) for v in grp],
-                    [float(v.tanfovy) for v in grp], H, W, sh_, rs.sh_degree, cps, rs.prefiltered, rs.debug,
-                    color_out=color[j:j + n], depth_out=depth[j:j + n])  # written in place
+                    rs.bg, s_m3, s_cp, s_op, s_sc, s_ro, rs.scale_modifier, s_cv, vm, pm, [float(v.tanfovx) for v in grp],
+                    [float(v.tanfovy) for v in grp], H, W, s_sh, rs.sh_degree, cps, rs.prefiltered, rs.debug,
+                    color_out=color[j:j + n], depth_out=depth[j:j + n], **extra)  # written in place
                 if keep_radii:
+                    per_view = r if counts is None else torch.split(r, counts[j:j + n])
                     for q in range(n):
-                        radii[j + q] = r[q]
+                        radii[j + q] = per_view[q]
                 return r
 
             with torch.no_grad():
@@ -383,7 +414,7 @@ def bind(_C) -> SimpleNamespace:
         with torch.no_grad():
             n_lanes = max(1, min(int(streams), B)) if dev.type == "cuda" else 1
             first = 0
-            if deferred and not _C.has_marks(m3.shape[0], W, H):
+            if deferred and counts is None and not _C.has_marks(m3.shape[0], W, H):
                 one(0, views[0], exact=True)  # a shape never seen before: one EXACT forward seeds its high-water marks
                 first = 1
             if n_lanes == 1:
@@ -417,7 +448,7 @@ def bind(_C) -> SimpleNamespace:
                 # the one host wait of the batch: every report has landed once the caller's stream is drained
                 torch.cuda.current_stream(dev).synchronize()
                 for j in range(first, B):
-                    _C.note_counts(m3.shape[0], W, H, reports[j])
+                    _C.note_counts(m3.shape[0] if counts is None else counts[j], W, H, reports[j])
                     if int(reports[j, 5]) != 0:
                         one(j, views[j], exact=True)
         return color, depth, radii

@@ -188,6 +188,18 @@ int brs_forward_views(const brs_view* views, int n_views, const brs_gaussians* g
                       float* out_color, float* out_depth, int* radii,
                       brs_alloc_fn alloc, void* alloc_ctx, long long* num_rendered,
                       const brs_fwd_options* opt, brs_stream stream);
+/* Extension: brs_forward_views where every view renders its OWN Gaussians (BloomScene's render loop, whose anchor
+ * culling and neural-Gaussian generation give each frame its own rows, bloomscene.py:174-219).  g holds the views'
+ * rows concatenated: view v owns rows [off_v, off_v + view_P[v]), off_v = view_P[0] + ... + view_P[v - 1], and
+ * g->P must equal the sum of view_P.  radii [g->P] in the same row order.  Each view's outputs are bit-identical to
+ * a brs_forward_ex of its own rows; a view with view_P[v] == 0 gets zeros without background, as that forward
+ * does.  view_P == NULL: every view sees all g->P rows (= brs_forward_views).  A negative entry or a sum other than
+ * g->P returns BRS_ERR_INVALID_ARG, a sum of 2^31 or more BRS_ERR_UNSUPPORTED, before any CUDA call.
+ * Limit: n_views * ceil(H / 16) < 65536. */
+int brs_forward_views_ex(const brs_view* views, int n_views, const brs_gaussians* g, const int* view_P,
+                         float* out_color, float* out_depth, int* radii,
+                         brs_alloc_fn alloc, void* alloc_ctx, long long* num_rendered,
+                         const brs_fwd_options* opt, brs_stream stream);
 /* Feeds the counts of a DEFERRED forward's report back into the high-water marks of its shape. */
 void brs_note_counts(int P, int image_width, int image_height, const uint32_t* report);
 /* High-water marks of a shape on the current device: returns 1 and fills out[3] = {R, R1, depth-key bits} if a
