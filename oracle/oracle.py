@@ -74,6 +74,8 @@ def lib():
         L.orc_backward.restype = C.c_int
         L.orc_backward_ex.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Grads)]
         L.orc_backward_ex.restype = C.c_int
+        L.orc_preprocess_backward.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Grads)]
+        L.orc_preprocess_backward.restype = C.c_int
         L.orc_set_f64_sums.argtypes = [C.c_int]
         L.orc_visible_filter.argtypes = [C.POINTER(_Inputs), C.c_int, C.c_void_p]
         L.orc_mark_visible.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -171,6 +173,22 @@ class Oracle:
                 self.L.orc_backward_ex(self.ctx, _ptr(d), _ptr(dd), C.byref(gs))
         finally:
             self.L.orc_set_f64_sums(0)
+        return g
+
+    def preprocess_backward(self, dL_dmeans2D, dL_dconic, dL_dcolors, dL_dz=None) -> Dict[str, np.ndarray]:
+        """The per-Gaussian stage of backward() alone, fed with arbitrary blend sums: dL_dmeans2D [P,3],
+        dL_dconic [P,4] (x, y, -, w; the reference's per-pair -0.5 included), dL_dcolors [P,3], dL_dz [P] or None (no
+        depth term).  Returns dL_dmeans3D, dL_dcov3D, dL_dsh, dL_dscales, dL_drotations (zeros where radii <= 0).
+        Call after forward()."""
+        P, M = self.P, self.M
+        ins = [_f32(np.asarray(a).reshape(P, k)) for a, k in ((dL_dmeans2D, 3), (dL_dconic, 4), (dL_dcolors, 3))]
+        dz = None if dL_dz is None else _f32(np.asarray(dL_dz).reshape(P))
+        g = {"dL_dmeans3D": np.zeros((P, 3), np.float32), "dL_dcov3D": np.zeros((P, 6), np.float32),
+             "dL_dsh": np.zeros((P, M, 3), np.float32), "dL_dscales": np.zeros((P, 3), np.float32),
+             "dL_drotations": np.zeros((P, 4), np.float32)}
+        gs = _Grads(*[_ptr(g[n]) if n in g and g[n].size else None for n, _ in _Grads._fields_])
+        if P:
+            self.L.orc_preprocess_backward(self.ctx, *[_ptr(a) for a in ins], _ptr(dz), C.byref(gs))
         return g
 
     def visible_filter(self, scales_stride: int = 3, **kw) -> np.ndarray:

@@ -873,6 +873,42 @@ static void cov3d_backward(const orc_ctx* c, int idx, const float* dL_dcov3Ds, f
 #undef MT
 }
 
+/* preprocessCUDA backward for every rendered Gaussian (rasterizer_impl.cu:476-503, backward.cu:144-396) from the
+ * per-Gaussian sums of the blend backward: dL_dmeans2D [P,3], dL_dconic [P,4] (x, y, -, w), dL_dcolors [P,3] and
+ * dL_dz [P] (NULL: no depth term).  Writes the rows with radii > 0 of g->dL_dmeans3D, dL_dcov3D, dL_dsh, dL_dscales
+ * and dL_drotations and leaves the other rows alone.  Call after orc_forward on the same ctx. */
+int orc_preprocess_backward(const orc_ctx* c, const float* dL_dmeans2D, const float* dL_dconic, const float* dL_dcolors,
+                            const float* dL_dz, const orc_grads* g)
+{
+	const int P = c->P;
+	const float* cov3D_all = c->cov3D_precomp ? c->cov3D_precomp : c->cov3D; /* rasterizer_impl.cu:481 */
+#pragma omp parallel for schedule(static)
+	for (int idx = 0; idx < P; idx++) {
+		if (!(c->radii[idx] > 0)) continue;
+		cov2d_backward(c, idx, cov3D_all + 6 * (size_t)idx, dL_dconic, g->dL_dmeans3D, g->dL_dcov3D);
+		/* preprocessCUDA backward (backward.cu:346-396) */
+		v3 m = V3(c->means3D[3 * idx], c->means3D[3 * idx + 1], c->means3D[3 * idx + 2]);
+		const float* proj = c->proj;
+		float hom[4];
+		transformPoint4x4(m, proj, hom);
+		float m_w = 1.0f / (hom[3] + 0.0000001f);
+		float mul1 = (proj[0] * m.x + proj[4] * m.y + proj[8] * m.z + proj[12]) * m_w * m_w;
+		float mul2 = (proj[1] * m.x + proj[5] * m.y + proj[9] * m.z + proj[13]) * m_w * m_w;
+		const float d2x = dL_dmeans2D[3 * idx], d2y = dL_dmeans2D[3 * idx + 1];
+		g->dL_dmeans3D[3 * idx] += (proj[0] * m_w - proj[3] * mul1) * d2x + (proj[1] * m_w - proj[3] * mul2) * d2y;
+		g->dL_dmeans3D[3 * idx + 1] += (proj[4] * m_w - proj[7] * mul1) * d2x + (proj[5] * m_w - proj[7] * mul2) * d2y;
+		g->dL_dmeans3D[3 * idx + 2] += (proj[8] * m_w - proj[11] * mul1) * d2x + (proj[9] * m_w - proj[11] * mul2) * d2y;
+		if (dL_dz) { /* z = p_view.z = view[2] x + view[6] y + view[10] z + view[14] (forward.cu:186,250) */
+			g->dL_dmeans3D[3 * idx] += c->view[2] * dL_dz[idx];
+			g->dL_dmeans3D[3 * idx + 1] += c->view[6] * dL_dz[idx];
+			g->dL_dmeans3D[3 * idx + 2] += c->view[10] * dL_dz[idx];
+		}
+		if (c->shs) sh_backward(c, idx, dL_dcolors, g->dL_dmeans3D, g->dL_dsh);
+		if (c->scales) cov3d_backward(c, idx, g->dL_dcov3D, g->dL_dscales, g->dL_drotations);
+	}
+	return 0;
+}
+
 /* Rasterizer::backward (rasterizer_impl.cu:403-504) after orc_forward on the same ctx.
  * All gradient arrays are zero-filled here like rasterize_points.cu:154-162. dL_dout_depth is unused. */
 int orc_backward_ex(orc_ctx* c, const float* dL_dpixels, const float* dL_ddepths, const orc_grads* g);
@@ -925,31 +961,7 @@ int orc_backward_ex(orc_ctx* c, const float* dL_dpixels, const float* dL_ddepths
 		for (size_t i = 0; i < (size_t)P; i++) dL_dz[i] = (float)s64.z[i];
 		free(s64.mean2D); free(s64.conic); free(s64.opacity); free(s64.colors); free(s64.z);
 	}
-	const float* cov3D_all = c->cov3D_precomp ? c->cov3D_precomp : c->cov3D; /* rasterizer_impl.cu:481 */
-#pragma omp parallel for schedule(static)
-	for (int idx = 0; idx < P; idx++) {
-		if (!(c->radii[idx] > 0)) continue;
-		cov2d_backward(c, idx, cov3D_all + 6 * (size_t)idx, dL_dconic, g->dL_dmeans3D, g->dL_dcov3D);
-		/* preprocessCUDA backward (backward.cu:346-396) */
-		v3 m = V3(c->means3D[3 * idx], c->means3D[3 * idx + 1], c->means3D[3 * idx + 2]);
-		const float* proj = c->proj;
-		float hom[4];
-		transformPoint4x4(m, proj, hom);
-		float m_w = 1.0f / (hom[3] + 0.0000001f);
-		float mul1 = (proj[0] * m.x + proj[4] * m.y + proj[8] * m.z + proj[12]) * m_w * m_w;
-		float mul2 = (proj[1] * m.x + proj[5] * m.y + proj[9] * m.z + proj[13]) * m_w * m_w;
-		const float d2x = g->dL_dmeans2D[3 * idx], d2y = g->dL_dmeans2D[3 * idx + 1];
-		g->dL_dmeans3D[3 * idx] += (proj[0] * m_w - proj[3] * mul1) * d2x + (proj[1] * m_w - proj[3] * mul2) * d2y;
-		g->dL_dmeans3D[3 * idx + 1] += (proj[4] * m_w - proj[7] * mul1) * d2x + (proj[5] * m_w - proj[7] * mul2) * d2y;
-		g->dL_dmeans3D[3 * idx + 2] += (proj[8] * m_w - proj[11] * mul1) * d2x + (proj[9] * m_w - proj[11] * mul2) * d2y;
-		if (dL_ddepths) { /* z = p_view.z = view[2] x + view[6] y + view[10] z + view[14] (forward.cu:186,250) */
-			g->dL_dmeans3D[3 * idx] += c->view[2] * dL_dz[idx];
-			g->dL_dmeans3D[3 * idx + 1] += c->view[6] * dL_dz[idx];
-			g->dL_dmeans3D[3 * idx + 2] += c->view[10] * dL_dz[idx];
-		}
-		if (c->shs) sh_backward(c, idx, g->dL_dcolors, g->dL_dmeans3D, g->dL_dsh);
-		if (c->scales) cov3d_backward(c, idx, g->dL_dcov3D, g->dL_dscales, g->dL_drotations);
-	}
+	orc_preprocess_backward(c, g->dL_dmeans2D, dL_dconic, g->dL_dcolors, dL_ddepths ? dL_dz : NULL, g);
 	free(dL_dconic);
 	free(dL_dz);
 	return 0;

@@ -80,7 +80,7 @@ def run_gpu(scene, cam, bg, dL_dpix, dL_ddepth=None, sh_degree=0):
 
 def check_public_outputs_are_slot_scalings(outs, accum, W, H):
     """preprocess_bwd.cu:163-167: dL_dmeans2D = (slot0 * (0.5f W), slot1 * (0.5f H), 0), dL_dopacity = slot5,
-    dL_dcolors = slots 6..8 (colours precomputed), bit for bit, for every rendered Gaussian; zeros otherwise."""
+    dL_dcolors = slots 6..8, bit for bit, for every rendered Gaussian; zeros otherwise."""
     f = np.float32
     vis = outs["radii"] > 0
     g = outs["grads"]
@@ -90,6 +90,8 @@ def check_public_outputs_are_slot_scalings(outs, accum, W, H):
     assert not m2[:, 2].any() and not m2[~vis].any()
     assert np.array_equal(g["dL_dopacity"][vis, 0], accum[vis, 5])
     assert not g["dL_dopacity"][~vis].any()
+    assert np.array_equal(g["dL_dcolors"][vis], accum[vis, 6:9])
+    assert not g["dL_dcolors"][~vis].any()
 
 
 def check_case(what, scene, cam, bg=BG, seed=0, depth="off", sh_degree=0, exclusions_allowed=0.0, report=None):
