@@ -731,12 +731,10 @@ int forward_impl(const brs_view* views, int n_views, const brs_gaussians* g, con
 	BRS_CUDA(cudaMemsetAsync(hdr, 0, HEADER_BYTES, stream));
 
 	PreprocessArgs pa{};
-	pa.P = P;
 	pa.D = view->sh_degree;
 	pa.M = g->shs ? view->sh_coeffs : 0;
 	pa.means3D = g->means3D;
 	pa.scales = g->scales;
-	pa.scale_modifier = view->scale_modifier;
 	pa.rotations = g->rotations;
 	pa.opacities = g->opacities;
 	pa.shs = g->shs;
@@ -758,45 +756,32 @@ int forward_impl(const brs_view* views, int n_views, const brs_gaussians* g, con
 	pa.records = reinterpret_cast<float4*>(c.geom + c.gl.records);
 	pa.depth_key = reinterpret_cast<uint32_t*>(c.geom + c.gl.depth_key);
 	pa.rect = reinterpret_cast<uint2*>(c.geom + c.gl.rect);
-	if (n_views == 1) {
-		pa.scale_modifier = view->scale_modifier;
-		pa.viewmatrix = view->viewmatrix;
-		pa.projmatrix = view->projmatrix;
-		pa.campos = view->campos;
-		pa.tan_fovx = view->tanfovx;
-		pa.tan_fovy = view->tanfovy;
-		pa.focal_y = H / (2.0f * view->tanfovy); // rasterizer_impl.cu:223-224
-		pa.focal_x = W / (2.0f * view->tanfovx);
-		pa.prefiltered = view->prefiltered;
-		pa.row_offset = 0;
-		BRS_STAGE(BRS_STAGE_PREPROCESS, launch_preprocess(pa, stream), debug, stream);
-	} else {
-		// one launch per 16 views: blockIdx.y picks the view, its outputs go to instances [v * P, (v + 1) * P), or
-		// with view_P to [off_v, off_v + view_P[v]), where off_v is also its first input row
-		size_t off = 0;
-		for (int v0 = 0; v0 < n_views; v0 += PreprocessViewTable::MAX_VIEWS) {
-			const int nv = n_views - v0 < PreprocessViewTable::MAX_VIEWS ? n_views - v0 : PreprocessViewTable::MAX_VIEWS;
-			PreprocessViewTable t{};
-			t.first_view = (uint32_t)v0;
-			for (int k = 0; k < nv; k++) {
-				const brs_view* vw = views + v0 + k;
-				PreprocessViewTable::Slot& sl = t.v[k];
-				sl.viewmatrix = vw->viewmatrix;
-				sl.projmatrix = vw->projmatrix;
-				sl.campos = vw->campos;
-				sl.tan_fovx = vw->tanfovx;
-				sl.tan_fovy = vw->tanfovy;
-				sl.focal_y = H / (2.0f * vw->tanfovy);
-				sl.focal_x = W / (2.0f * vw->tanfovx);
-				sl.scale_modifier = vw->scale_modifier;
-				sl.prefiltered = vw->prefiltered;
-				sl.count = (uint32_t)(view_P != nullptr ? view_P[v0 + k] : P);
-				sl.row = view_P != nullptr ? (uint32_t)off : 0u;
-				sl.inst = (uint32_t)off;
-				off += sl.count;
-			}
-			BRS_STAGE(BRS_STAGE_PREPROCESS, launch_preprocess_stack(pa, t, nv, stream), debug, stream);
+	// one launch per MAX_VIEWS views: blockIdx.y picks the view, its outputs go to instances [v * P, (v + 1) * P), or
+	// with view_P to [off_v, off_v + view_P[v]), where off_v is also its first input row.  A single view is the
+	// table {(0, 0, P)}.
+	size_t off = 0;
+	for (int v0 = 0; v0 < n_views; v0 += PreprocessViewTable::MAX_VIEWS) {
+		const int nv = n_views - v0 < PreprocessViewTable::MAX_VIEWS ? n_views - v0 : PreprocessViewTable::MAX_VIEWS;
+		PreprocessViewTable t{};
+		t.first_view = (uint32_t)v0;
+		for (int k = 0; k < nv; k++) {
+			const brs_view* vw = views + v0 + k;
+			PreprocessViewTable::Slot& sl = t.v[k];
+			sl.viewmatrix = vw->viewmatrix;
+			sl.projmatrix = vw->projmatrix;
+			sl.campos = vw->campos;
+			sl.tan_fovx = vw->tanfovx;
+			sl.tan_fovy = vw->tanfovy;
+			sl.focal_y = H / (2.0f * vw->tanfovy); // rasterizer_impl.cu:223-224
+			sl.focal_x = W / (2.0f * vw->tanfovx);
+			sl.scale_modifier = vw->scale_modifier;
+			sl.prefiltered = vw->prefiltered;
+			sl.count = (uint32_t)(view_P != nullptr ? view_P[v0 + k] : P);
+			sl.row = view_P != nullptr ? (uint32_t)off : 0u;
+			sl.inst = (uint32_t)off;
+			off += sl.count;
 		}
+		BRS_STAGE(BRS_STAGE_PREPROCESS, launch_preprocess(pa, t, nv, stream), debug, stream);
 	}
 
 	// ---- deferred: the caller's capacities (or the high-water marks), no host wait at all ----

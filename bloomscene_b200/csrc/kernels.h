@@ -9,39 +9,33 @@ namespace brs {
 void count_launch();
 
 // ---- preprocess.cu ------------------------------------------------------------------------------
+// What every view of a launch shares: the input and output base pointers (a view's slot says where its rows and
+// instances start), the SH layout and the image size.
 struct PreprocessArgs {
-	int P, D, M;
+	int D, M;
 	const float* means3D;
 	const float* scales;
-	float scale_modifier;
 	const float* rotations;
 	const float* opacities;
 	const float* shs;
 	const float* cov3D_precomp;
 	const float* colors_precomp;
-	const float* viewmatrix;
-	const float* projmatrix;
-	const float* campos;
 	int W, H;
-	float tan_fovx, tan_fovy, focal_x, focal_y;
 	uint32_t grid_x, grid_y;
-	int prefiltered;
 	int eager_sh;         // request every Gaussian's SH row up front (most are visible) instead of the visible ones' later
-	uint32_t row_offset;  // tile rows added to the rectangle: this view's place in a stack of views (brs_forward_views), else 0
-	// outputs
+	// outputs, indexed by instance
 	int* radii;
-	float4* records;      // [3P]
-	uint32_t* depth_key;  // [P]
-	uint2* rect;          // [P]
+	float4* records;      // [3 * instances]
+	uint32_t* depth_key;  // [instances]
+	uint2* rect;          // [instances]
 	uint32_t* total_tiles; // [5], pre-zeroed: R = tile instances, R1 = supertile instances, max(~depth bits),
 	                       // max(depth bits) over visible, V = number of visible Gaussians
 };
-cudaError_t launch_preprocess(const PreprocessArgs& a, cudaStream_t stream); // one view of a.P Gaussians
-// Up to MAX_VIEWS views of a stack in one launch: the per-view fields of PreprocessArgs come from the table,
-// view k of the launch is view first_view + k of the stack (tile row offset).  View k reads input rows
-// [row, row + count) and writes instances [inst, inst + count); PreprocessArgs::P is not read by the kernel.
-// A single view is the table {(0, 0, P)}, a stack of one Gaussian set {(0, v * P, P)}, a stack whose views
-// own consecutive rows of concatenated inputs (brs_forward_views_ex) {(off_v, off_v, P_v)}.
+// Up to MAX_VIEWS views in one launch, each described by its slot alone: its camera, and the count Gaussians it
+// reads from input rows [row, row + count) and writes to instances [inst, inst + count).  View k of the launch
+// is view first_view + k of the stack, which places its tile rows.  A single view is the table {(0, 0, P)}, a
+// stack of one Gaussian set {(0, v * P, P)}, a stack whose views own consecutive rows of concatenated inputs
+// (brs_forward_views_ex) {(off_v, off_v, P_v)}.
 struct PreprocessViewTable {
 	static constexpr int MAX_VIEWS = 16;
 	struct Slot {
@@ -54,7 +48,7 @@ struct PreprocessViewTable {
 	} v[MAX_VIEWS];
 	uint32_t first_view;
 };
-cudaError_t launch_preprocess_stack(const PreprocessArgs& a, const PreprocessViewTable& t, int n_views, cudaStream_t stream);
+cudaError_t launch_preprocess(const PreprocessArgs& a, const PreprocessViewTable& t, int n_views, cudaStream_t stream);
 
 struct FilterArgs {
 	int P;

@@ -200,7 +200,7 @@ __device__ __forceinline__ void stage_camera(float* s_cam, const float* view, co
 //   the visible Gaussians are requested, after the geometry phase.  The host picks EAGER when the last views
 //   of this shape had most Gaussians visible (the rows of culled Gaussians are wasted traffic).
 template <bool VEC, bool EAGER>
-__device__ __forceinline__ void preprocess_body(const PreprocessArgs& a)
+__device__ __forceinline__ void preprocess_body(const PreprocessArgs& a, const PreprocessViewTable::Slot& v, uint32_t row_offset)
 {
 	extern __shared__ float4 s_dyn[]; // SH staging (only when a.shs != nullptr)
 	__shared__ float s_cam[36];
@@ -210,7 +210,8 @@ __device__ __forceinline__ void preprocess_body(const PreprocessArgs& a)
 	const int block_first = blockIdx.x * PRE_THREADS;
 	const int idx = block_first + threadIdx.x;
 	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-	const bool in_range = idx < a.P;
+	const int P = (int)v.count;
+	const bool in_range = idx < P;
 	const bool bulk = VEC && a.shs != nullptr;
 
 	if (bulk) {
@@ -219,9 +220,9 @@ __device__ __forceinline__ void preprocess_body(const PreprocessArgs& a)
 		__syncwarp();
 		if (EAGER) {
 			// even lanes fetch their own row and their neighbour's (one 384-byte copy; 192 at the end of the array)
-			const uint32_t rows = (uint32_t)max(0, min(32, a.P - (block_first + 32 * warp)));
+			const uint32_t rows = (uint32_t)max(0, min(32, P - (block_first + 32 * warp)));
 			if (in_range && !(lane & 1))
-				bulk_copy_g2s(s_dyn + sh_row_slot(threadIdx.x), a.shs + (size_t)idx * 48, idx + 1 < a.P ? 384u : 192u, &s_bar[warp]);
+				bulk_copy_g2s(s_dyn + sh_row_slot(threadIdx.x), a.shs + (size_t)idx * 48, idx + 1 < P ? 384u : 192u, &s_bar[warp]);
 			if (lane == 0)
 				mbar_arrive_expect_tx(&s_bar[warp], 192u * rows);
 		}
@@ -230,10 +231,10 @@ __device__ __forceinline__ void preprocess_body(const PreprocessArgs& a)
 	GeomInputs in;
 	float opacity = 0.f;
 	if (in_range) {
-		in = load_geom_inputs(a.means3D, a.scales, 3, a.rotations, a.cov3D_precomp, idx, a.scale_modifier);
+		in = load_geom_inputs(a.means3D, a.scales, 3, a.rotations, a.cov3D_precomp, idx, v.scale_modifier);
 		opacity = __ldg(a.opacities + idx);
 	}
-	stage_camera(s_cam, a.viewmatrix, a.projmatrix, a.campos);
+	stage_camera(s_cam, v.viewmatrix, v.projmatrix, v.campos);
 	__syncthreads();
 	const float* view = s_cam;
 	const float* proj = s_cam + 16;
@@ -243,15 +244,15 @@ __device__ __forceinline__ void preprocess_body(const PreprocessArgs& a)
 	float3 p_orig = {0.f, 0.f, 0.f};
 	if (in_range) {
 		p_orig = in.mean;
-		visible = compute_geometry(in, view, proj, a.W, a.H, a.tan_fovx, a.tan_fovy, a.focal_x, a.focal_y, a.grid_x,
-		                           a.grid_y, a.prefiltered != 0, g);
+		visible = compute_geometry(in, view, proj, a.W, a.H, v.tan_fovx, v.tan_fovy, v.focal_x, v.focal_y, a.grid_x,
+		                           a.grid_y, v.prefiltered != 0, g);
 	}
 
 	const uint32_t vis_mask = __ballot_sync(0xffffffffu, visible);
 	uint32_t tiles = 0u, cells = 0u; // tile / supertile instances of this Gaussian
 	if (visible) {
-		g.rect_min.y += a.row_offset; // the view's place in a stack of views (0 for a single view)
-		g.rect_max.y += a.row_offset;
+		g.rect_min.y += row_offset; // the view's place in a stack of views (0 for a single view)
+		g.rect_max.y += row_offset;
 		tiles = (g.rect_max.y - g.rect_min.y) * (g.rect_max.x - g.rect_min.x);
 		cells = ((((g.rect_max.x - 1) >> ST_SHIFT) + 1) - (g.rect_min.x >> ST_SHIFT)) *
 		        ((((g.rect_max.y - 1) >> ST_SHIFT) + 1) - (g.rect_min.y >> ST_SHIFT));
@@ -268,7 +269,7 @@ __device__ __forceinline__ void preprocess_body(const PreprocessArgs& a)
 			if (!EAGER) {
 				// a pair of rows is fetched (by its even lane) when either of its Gaussians is visible
 				const uint32_t pair_mask = (vis_mask | (vis_mask >> 1)) & 0x55555555u;
-				const uint32_t short_pair = (in_range && !(lane & 1) && idx + 1 >= a.P && ((pair_mask >> lane) & 1u)) ? 1u : 0u;
+				const uint32_t short_pair = (in_range && !(lane & 1) && idx + 1 >= P && ((pair_mask >> lane) & 1u)) ? 1u : 0u;
 				if (in_range && ((pair_mask >> lane) & 1u))
 					bulk_copy_g2s(s_dyn + sh_row_slot(threadIdx.x), a.shs + (size_t)idx * 48, short_pair ? 192u : 384u, &s_bar[warp]);
 				const uint32_t shorts = __popc(__ballot_sync(0xffffffffu, short_pair != 0u));
@@ -308,7 +309,7 @@ __device__ __forceinline__ void preprocess_body(const PreprocessArgs& a)
 	}
 
 	// ---- outputs ----
-	if (idx < a.P) {
+	if (idx < P) {
 		if (visible) {
 			const float tau = cull_tau(g.conic, opacity, g.radius);
 			float4* rec = a.records + 3 * (size_t)idx;
@@ -374,11 +375,10 @@ __device__ __forceinline__ const float* view_rows(const float* p, size_t floats)
 template <bool VEC, bool EAGER>
 __global__ void __launch_bounds__(PRE_THREADS) preprocess_kernel(PreprocessArgs a, PreprocessViewTable t)
 {
-	const PreprocessViewTable::Slot& v = t.v[blockIdx.y];
+	const PreprocessViewTable::Slot v = t.v[blockIdx.y];
 	if (blockIdx.x * PRE_THREADS >= v.count)
 		return;
 	const size_t row = v.row, first = v.inst;
-	a.P = (int)v.count;
 	a.means3D += 3 * row;
 	a.scales = view_rows(a.scales, 3 * row);
 	a.rotations = view_rows(a.rotations, 4 * row);
@@ -386,21 +386,12 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_kernel(PreprocessArgs 
 	a.shs = view_rows(a.shs, (size_t)(3 * a.M) * row);
 	a.cov3D_precomp = view_rows(a.cov3D_precomp, 6 * row);
 	a.colors_precomp = view_rows(a.colors_precomp, 3 * row);
-	a.viewmatrix = v.viewmatrix;
-	a.projmatrix = v.projmatrix;
-	a.campos = v.campos;
-	a.tan_fovx = v.tan_fovx;
-	a.tan_fovy = v.tan_fovy;
-	a.focal_x = v.focal_x;
-	a.focal_y = v.focal_y;
-	a.scale_modifier = v.scale_modifier;
-	a.prefiltered = v.prefiltered;
-	a.row_offset += (t.first_view + blockIdx.y) * a.grid_y;
 	a.radii += first;
 	a.records += 3 * first;
 	a.depth_key += first;
 	a.rect += first;
-	preprocess_body<VEC, EAGER>(a);
+	const uint32_t row_offset = (t.first_view + blockIdx.y) * a.grid_y;
+	preprocess_body<VEC, EAGER>(a, v, row_offset);
 }
 
 // ---- K10 ----------------------------------------------------------------------------------------
@@ -520,29 +511,10 @@ __global__ void __launch_bounds__(256)
 
 // ---- launchers ----------------------------------------------------------------------------------
 
-cudaError_t launch_preprocess(const PreprocessArgs& a, cudaStream_t stream)
-{
-	PreprocessViewTable t{};
-	PreprocessViewTable::Slot& s = t.v[0];
-	s.viewmatrix = a.viewmatrix;
-	s.projmatrix = a.projmatrix;
-	s.campos = a.campos;
-	s.tan_fovx = a.tan_fovx;
-	s.tan_fovy = a.tan_fovy;
-	s.focal_x = a.focal_x;
-	s.focal_y = a.focal_y;
-	s.scale_modifier = a.scale_modifier;
-	s.prefiltered = a.prefiltered;
-	s.row = 0;
-	s.inst = 0;
-	s.count = a.P < 0 ? 0u : (uint32_t)a.P;
-	return launch_preprocess_stack(a, t, 1, stream);
-}
-
 // The grid is sized by the largest view of the launch (not a flat grid over all rows with a per-block search of
 // the table): the block -> (view, row) map stays blockIdx.y / blockIdx.x * PRE_THREADS as for a single view, at
 // the price of blocks that exit at once in the shorter views of a ragged stack.
-cudaError_t launch_preprocess_stack(const PreprocessArgs& a, const PreprocessViewTable& t, int n_views, cudaStream_t stream)
+cudaError_t launch_preprocess(const PreprocessArgs& a, const PreprocessViewTable& t, int n_views, cudaStream_t stream)
 {
 	if (n_views <= 0)
 		return cudaSuccess;
